@@ -3,11 +3,14 @@
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                   (the reference's CPU path on the host cores)
+    python bench.py ... --dump-outputs DIR                 (also writes the last timed step's results as .npy files)
 
 One "step" = one pass of the hot path over one batch: Injector (n_levels=3) forward+backward and
 Extractor (n_levels=1) forward+backward at the ViT-Adapter shape named in `config.workload`
 (BASELINE.json configs[1]: ViT-Adapter-B, 512x512, 16 images per GPU, fp32 by default).
 metric = sampled points per second (Gsamples/s), pts = N*Lq*M*L*P, whole job over all GPUs.
+--steps K sets the timed region of that metric: exactly K steps on device-resident inputs. The informational arms clamp
+it: `e2e` times 5 passes of min(max(K, 4), 50) steps and `ref_cuda` min(max(K, 2), 10) steps; both report their count.
 
 Printed: ONE JSON line on stdout (rank 0). Keys follow the driver contract plus `roofline`,
 `cpu_baseline`, `e2e`, `clocks`, `gpu_launches`, and informational `kernels` / `ref_cuda`.
@@ -260,6 +263,32 @@ def workload_config(variant, batch, dtype):
     }
 
 
+DUMP_ELEMS = 1 << 20   # per array: the 8 float32 arrays of an Injector+Extractor step stay below 64 MB in all
+
+
+def dump_positions(n):
+    """The flattened positions dump_outputs writes of an array of n > DUMP_ELEMS elements: one at a seeded random place in
+    each of DUMP_ELEMS equal stretches, in order. They depend on n alone, so every run with the same arguments samples the
+    same elements."""
+    lo = torch.arange(DUMP_ELEMS + 1, dtype=torch.int64) * n // DUMP_ELEMS
+    u = torch.rand(DUMP_ELEMS, generator=torch.Generator().manual_seed(0), dtype=torch.float64)
+    return lo[:-1] + (u * (lo[1:] - lo[:-1])).long()
+
+
+def dump_outputs(directory, names, results):
+    """Write each call's (out, grad_value, grad_loc, grad_aw) as <directory>/<call>_<array>.npy in float32: the whole
+    flattened array, or for one of more than DUMP_ELEMS elements its elements at dump_positions(), so that two builds can
+    be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, arrays in zip(names, results):
+        for what, t in zip(('out', 'grad_value', 'grad_loc', 'grad_aw'), arrays):
+            flat = t.detach().reshape(-1)
+            if flat.numel() > DUMP_ELEMS:
+                flat = flat[dump_positions(flat.numel()).to(flat.device)]
+            np.save(os.path.join(directory, '%s_%s.npy' % (name, what)), flat.float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------
@@ -309,18 +338,28 @@ def run_ours(args):
         pts_step += calls[-1]['pts']
     torch.cuda.synchronize()
 
-    def step_device(events=None):
-        """One step on device-resident inputs, straight through the C-ABI binding."""
+    def step_device(events=None, keep=False):
+        """One step on device-resident inputs, straight through the C-ABI binding. With keep, returns per call what a
+        caller of the binding receives: [out, grad_value, grad_loc, grad_aw]; otherwise every result is freed as soon as
+        it is returned, so its memory serves the next allocation of the step."""
+        results = []
         for ci, c in enumerate(calls):
             d = c['dev']
             if events is not None:
                 events[ci][0].record()
-            _cabi.forward(d['value'], d['shapes'], d['lsi'], d['loc'], d['aw'], 64)
+            out = _cabi.forward(d['value'], d['shapes'], d['lsi'], d['loc'], d['aw'], 64)
+            if keep:
+                results.append([out])
+            del out
             if events is not None:
                 events[ci][1].record()
-            _cabi.backward(d['value'], d['shapes'], d['lsi'], d['loc'], d['aw'], d['grad_out'], 64)
+            grads = _cabi.backward(d['value'], d['shapes'], d['lsi'], d['loc'], d['aw'], d['grad_out'], 64)
+            if keep:
+                results[-1].extend(grads)
+            del grads
             if events is not None:
                 events[ci][2].record()
+        return results
 
     def barrier():
         if world > 1:
@@ -328,8 +367,11 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     # ---- warm-up -------------------------------------------------------------------------------------------
-    for _ in range(args.warmup):
-        step_device()
+    # --dump-outputs keeps the results of the last timed step; the last warm-up step keeps its own too, so the caching
+    # allocator already holds the memory that step needs and the timed region allocates none
+    dumping = bool(args.dump_outputs)
+    for w in range(args.warmup):
+        step_device(keep=dumping and w == args.warmup - 1)
     barrier()
 
     # ---- timed region: exactly K steps, CUDA events, per-kernel events inside ------------------------------
@@ -345,13 +387,16 @@ def run_ours(args):
     t0 = time.time()
     e0.record()
     for k in range(K):
-        step_device(ev[k])
+        last = step_device(ev[k], keep=dumping and k == K - 1)
     e1.record()
     barrier()
     t1 = time.time()
     launches = _cabi.launch_count() - launches0
     elapsed_ms = e0.elapsed_time(e1)
     clocks = sampler.stop(t0, t1) if sampler else None
+    if rank == 0 and dumping:
+        dump_outputs(args.dump_outputs, [c['name'] for c in calls], last)
+    del last
 
     # per-kernel average durations (fwd: events 0->1, bwd: events 1->2; bwd includes its grad_value zero-fill)
     kernels = []
@@ -420,7 +465,7 @@ def run_ours(args):
 
     h2d = sum(sum(c['host'][k].numel() * c['host'][k].element_size() for k in in_keys) for c in calls)
     d2h = sum(sum(t.numel() * t.element_size() for t in bufs) for bufs in host_out[0])
-    e2e_steps = max(4, min(K, 50))   # the timed region includes the pipeline's fill and drain: all K steps, like the device arm
+    e2e_steps = max(4, min(K, 50))   # per pass; each pass includes the pipeline's fill and drain, five passes are timed
     # warm-up: W steps, then one full untimed pass of the same length as the timed ones (the first pass after the
     # device-resident phase was 3.5x slower than the following ones in round 1: pinned result buffers touched for the first
     # time by the DMA engine and the copy streams' first use all land in it)
@@ -467,7 +512,7 @@ def run_ours(args):
                 rms = r0.elapsed_time(r1) / nref
                 ref_cuda = {'what': "reference's own CUDA kernels (ms_deform_im2col_cuda.cuh) recompiled for sm_100a, fp32, "
                                     'same inputs, 1 GPU', 'ms_per_step': rms, 'value': pts_step / (rms * 1e-3) / 1e9,
-                            'unit': 'Gsamples/s'}
+                            'unit': 'Gsamples/s', 'steps': nref}
                 del f32
         except Exception as e:  # informational only
             ref_cuda = {'error': repr(e)}
@@ -754,7 +799,8 @@ def main():
     _GUARD = _StdoutGuard()
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20,
+                    help='timed steps of the headline metric (the e2e arm clamps to 4..50 per pass, ref_cuda to 2..10)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--variant', default='B', choices=sorted(VARIANTS))
@@ -764,7 +810,13 @@ def main():
     ap.add_argument('--no-ref-cuda', action='store_true')
     ap.add_argument('--no-other-shapes', action='store_true')
     ap.add_argument('--no-step', action='store_true', help='skip the model-level training-step block (bench_step.step_bench)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed (rank 0) as DIR/<call>_<array>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs records the GPU path (--impl ours)')
     if args.warmup < 3 and args.impl == 'ours':
         args.warmup = 3
     if args.impl == 'reference':

@@ -1,5 +1,5 @@
-import cProfile, pstats, sys, io
-sys.path.insert(0, '/root/repo')
+import cProfile, pstats, sys, io, os
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import vit_adapter_b200 as vab
 from vit_adapter_b200.adapter import InteractionBlock, deform_inputs
