@@ -180,6 +180,15 @@ def _stream():
     return ctypes.c_void_p(torch._C._cuda_getCurrentRawStream(torch.cuda.current_device()))
 
 
+def _workspace(nbytes, dev):
+    """(buffer, pointer) of `nbytes` bytes of device scratch for one call, or (None, None) when none is needed. Keep the
+    buffer referenced until the call has been issued."""
+    if not nbytes:
+        return None, None
+    ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+    return ws, ws.data_ptr()
+
+
 class TensorMemo:
     """Memo keyed by tensor IDENTITY (weak reference) + version counter. Keying by data_ptr would be wrong: the
     caching allocator hands a freed address to the next tensor of the same size, with different contents."""
@@ -276,12 +285,11 @@ def backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight
         grad_loc = torch.empty_like(sampling_loc)
         grad_aw = torch.empty_like(attn_weight)
         ws_bytes = lib.msda_backward_workspace_bytes(ctypes.byref(dims), code)
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+        ws, ws_ptr = _workspace(ws_bytes, dev)
         rc = lib.msda_backward(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
                                level_start_index.data_ptr(), sampling_loc.data_ptr(), attn_weight.data_ptr(),
                                grad_output.data_ptr(), grad_value.data_ptr(), grad_loc.data_ptr(),
-                               grad_aw.data_ptr(), ws.data_ptr() if ws is not None else None, ws_bytes,
-                               _stream())
+                               grad_aw.data_ptr(), ws_ptr, ws_bytes, _stream())
     if rc != 0:
         _raise(rc, 'ms_deform_attn_backward')
     return grad_value, grad_loc, grad_aw
@@ -324,22 +332,61 @@ def _fused_dims(value, reference_points, sampling_offsets, attn_logits):
     return MsdaDims(N, S, M, D, L, Lq, P), int(reference_points.shape[0]), int(reference_points.shape[2])
 
 
-def forward_fused(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits):
-    """out [N, Lq, M*D] from RAW offsets / logits: softmax and location arithmetic happen inside the kernel."""
-    lib = load()
-    dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
-                      reference_points=reference_points, sampling_offsets=sampling_offsets, attn_logits=attn_logits)
-    dims, rb, rl = _fused_dims(value, reference_points, sampling_offsets, attn_logits)
+def _forward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, offsets, logits, row_stride):
+    """out [N, Lq, M*D] of the fused entry. `row_stride`: floats between consecutive (b, q) rows of `offsets` and `logits`,
+    0 = dense. Runs under the caller's device guard."""
     _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
-    code = _DTYPES.get(value.dtype)
-    with _on(dev):
-        out = torch.empty((dims.batch, dims.num_query, dims.num_heads * dims.channels), dtype=value.dtype, device=dev)
-        rc = lib.msda_forward_fused(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
-                                    level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl,
-                                    sampling_offsets.data_ptr(), attn_logits.data_ptr(), 0, 0, out.data_ptr(), _stream())
+    out = torch.empty((dims.batch, dims.num_query, dims.num_heads * dims.channels), dtype=value.dtype, device=value.device)
+    rc = load().msda_forward_fused(ctypes.byref(dims), _DTYPES.get(value.dtype), value.data_ptr(), spatial_shapes.data_ptr(),
+                                   level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl, offsets.data_ptr(),
+                                   logits.data_ptr(), row_stride, row_stride, out.data_ptr(), _stream())
     if rc != 0:
         _raise(rc, 'msda_forward_fused')
     return out
+
+
+def _backward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, offsets, logits, row_stride,
+                    grad_output, grad_offsets, grad_logits):
+    """grad_value of the fused entry; writes the offset and logit gradients into `grad_offsets` / `grad_logits`, which have
+    the row stride of `offsets` / `logits`. Runs under the caller's device guard."""
+    _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
+    if grad_output.dtype != value.dtype:
+        raise RuntimeError('grad_output dtype %s != value dtype %s' % (grad_output.dtype, value.dtype))
+    lib = load()
+    code = _DTYPES.get(value.dtype)
+    grad_value = torch.empty_like(value)
+    ws_bytes = lib.msda_backward_workspace_bytes(ctypes.byref(dims), code)
+    ws, ws_ptr = _workspace(ws_bytes, value.device)
+    rc = lib.msda_backward_fused(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
+                                 level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl, offsets.data_ptr(),
+                                 logits.data_ptr(), row_stride, row_stride, grad_output.data_ptr(), grad_value.data_ptr(),
+                                 grad_offsets.data_ptr(), grad_logits.data_ptr(), ws_ptr, ws_bytes, _stream())
+    if rc != 0:
+        _raise(rc, 'msda_backward_fused')
+    return grad_value
+
+
+def forward_fused(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits):
+    """out [N, Lq, M*D] from RAW offsets / logits: softmax and location arithmetic happen inside the kernel."""
+    dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
+                      reference_points=reference_points, sampling_offsets=sampling_offsets, attn_logits=attn_logits)
+    dims, rb, rl = _fused_dims(value, reference_points, sampling_offsets, attn_logits)
+    with _on(dev):
+        return _forward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, sampling_offsets,
+                              attn_logits, 0)
+
+
+def backward_fused(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits, grad_output):
+    """(grad_value, grad_sampling_offsets, grad_attn_logits) of the fused entry."""
+    dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
+                      reference_points=reference_points, sampling_offsets=sampling_offsets, attn_logits=attn_logits,
+                      grad_output=grad_output)
+    dims, rb, rl = _fused_dims(value, reference_points, sampling_offsets, attn_logits)
+    with _on(dev):
+        grad_off, grad_logits = torch.empty_like(sampling_offsets), torch.empty_like(attn_logits)
+        grad_value = _backward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points,
+                                     sampling_offsets, attn_logits, 0, grad_output, grad_off, grad_logits)
+    return grad_value, grad_off, grad_logits
 
 
 def _merged_dims(value, reference_points, merged, n_levels, n_points):
@@ -358,75 +405,27 @@ def forward_fused_merged(value, spatial_shapes, level_start_index, reference_poi
     """Fused forward reading offsets and logits from ONE buffer [N, Lq, M*L*P*3] — the output of a single GEMM whose
     weight is cat(sampling_offsets.weight, attention_weights.weight): columns [0, M*L*P*2) are the raw offsets,
     columns [M*L*P*2, M*L*P*3) the raw logits."""
-    lib = load()
     dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
                       reference_points=reference_points, merged=merged)
     dims, rb, rl, width = _merged_dims(value, reference_points, merged, n_levels, n_points)
-    _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
-    code = _DTYPES.get(value.dtype)
+    split = width // 3 * 2
     with _on(dev):
-        out = torch.empty((dims.batch, dims.num_query, dims.num_heads * dims.channels), dtype=value.dtype, device=dev)
-        rc = lib.msda_forward_fused(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
-                                    level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl,
-                                    merged.data_ptr(), merged.data_ptr() + 4 * (width // 3) * 2, width, width,
-                                    out.data_ptr(), _stream())
-    if rc != 0:
-        _raise(rc, 'msda_forward_fused')
-    return out
+        return _forward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, merged[..., :split],
+                              merged[..., split:], width)
 
 
 def backward_fused_merged(value, spatial_shapes, level_start_index, reference_points, merged, n_levels, n_points, grad_output):
     """(grad_value, grad_merged): grad_merged has the layout of `merged`, i.e. it is the merged GEMM's output gradient."""
-    lib = load()
     dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
                       reference_points=reference_points, merged=merged, grad_output=grad_output)
     dims, rb, rl, width = _merged_dims(value, reference_points, merged, n_levels, n_points)
-    _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
-    code = _DTYPES.get(value.dtype)
-    if grad_output.dtype != value.dtype:
-        raise RuntimeError('grad_output dtype %s != value dtype %s' % (grad_output.dtype, value.dtype))
+    split = width // 3 * 2
     with _on(dev):
-        grad_value = torch.empty_like(value)
         grad_merged = torch.empty_like(merged)
-        ws_bytes = lib.msda_backward_workspace_bytes(ctypes.byref(dims), code)
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
-        off_logits = 4 * (width // 3) * 2
-        rc = lib.msda_backward_fused(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
-                                     level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl,
-                                     merged.data_ptr(), merged.data_ptr() + off_logits, width, width,
-                                     grad_output.data_ptr(), grad_value.data_ptr(), grad_merged.data_ptr(),
-                                     grad_merged.data_ptr() + off_logits,
-                                     ws.data_ptr() if ws is not None else None, ws_bytes, _stream())
-    if rc != 0:
-        _raise(rc, 'msda_backward_fused')
+        grad_value = _backward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points,
+                                     merged[..., :split], merged[..., split:], width, grad_output,
+                                     grad_merged[..., :split], grad_merged[..., split:])
     return grad_value, grad_merged
-
-
-def backward_fused(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits, grad_output):
-    """(grad_value, grad_sampling_offsets, grad_attn_logits) of the fused entry."""
-    lib = load()
-    dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
-                      reference_points=reference_points, sampling_offsets=sampling_offsets, attn_logits=attn_logits,
-                      grad_output=grad_output)
-    dims, rb, rl = _fused_dims(value, reference_points, sampling_offsets, attn_logits)
-    _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
-    code = _DTYPES.get(value.dtype)
-    if grad_output.dtype != value.dtype:
-        raise RuntimeError('grad_output dtype %s != value dtype %s' % (grad_output.dtype, value.dtype))
-    with _on(dev):
-        grad_value = torch.empty_like(value)
-        grad_off = torch.empty_like(sampling_offsets)
-        grad_logits = torch.empty_like(attn_logits)
-        ws_bytes = lib.msda_backward_workspace_bytes(ctypes.byref(dims), code)
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
-        rc = lib.msda_backward_fused(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
-                                     level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl,
-                                     sampling_offsets.data_ptr(), attn_logits.data_ptr(), 0, 0, grad_output.data_ptr(),
-                                     grad_value.data_ptr(), grad_off.data_ptr(), grad_logits.data_ptr(),
-                                     ws.data_ptr() if ws is not None else None, ws_bytes, _stream())
-    if rc != 0:
-        _raise(rc, 'msda_backward_fused')
-    return grad_value, grad_off, grad_logits
 
 
 def dwconv_supported(x, weight, H, W):
@@ -466,9 +465,9 @@ def dwconv_backward(x, weight, grad_y, H, W, need_input=True, need_weight=True):
             gw = torch.empty((C, 1, 3, 3), dtype=adt, device=dev)
             gb = torch.empty((C,), dtype=adt, device=dev)
             ws_bytes = lib.adapter_dwconv_backward_weight_workspace_bytes(code, B, n, C, H, W)
-            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+            ws, ws_ptr = _workspace(ws_bytes, dev)
             rc = lib.adapter_dwconv_backward_weight(code, x.data_ptr(), grad_y.data_ptr(), gw.data_ptr(), gb.data_ptr(),
-                                                    B, n, C, H, W, ws.data_ptr() if ws is not None else None, ws_bytes, _stream())
+                                                    B, n, C, H, W, ws_ptr, ws_bytes, _stream())
             if rc != 0:
                 _raise(rc, 'adapter_dwconv_backward_weight')
             gw, gb = gw.to(weight.dtype), gb.to(weight.dtype)

@@ -78,9 +78,23 @@ static int fail(int code, const char* fmt, ...) {
   return code;
 }
 
-static int cuda_fail(cudaError_t e, const char* what) {
+static int cuda_fail(cudaError_t e, const char* fmt, ...) {
+  char what[256];
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(what, sizeof(what), fmt, ap);
+  va_end(ap);
   snprintf(g_err, sizeof(g_err), "%s: %s (%s)", what, cudaGetErrorString(e), cudaGetErrorName(e));
   return (int)e;
+}
+
+// 0, or the return code of a failed launch
+static int launched(cudaError_t e, const char* what) { return e == cudaSuccess ? 0 : cuda_fail(e, "%s", what); }
+
+// The fused launchers return cudaErrorNotSupported when they have no kernel for G.
+static int fused_launched(cudaError_t e, const char* who, int G) {
+  if (e == cudaErrorNotSupported) return fail(MSDA_E_UNSUPPORTED, "%s: no fused kernel for G=%d", who, G);
+  return e == cudaSuccess ? 0 : cuda_fail(e, "%s launch", who);
 }
 
 static size_t elem_size(int dtype) {
@@ -270,10 +284,67 @@ static bool plan_cell(const msda_dims* d, int dtype, Params& p, CellPlan* cp) {
   return false;
 }
 
-static void fill_params(Params& p, const msda_dims* d) {
+// The dims and the inputs every entry point has (for the fused ones `loc` / `aw` are the raw offsets / logits)
+static void fill_params(Params& p, const msda_dims* d, const void* value, const int64_t* shapes, const int64_t* lsi,
+                        const void* loc, const void* aw) {
   memset(&p, 0, sizeof(p));
   p.N = d->batch; p.S = d->spatial_size; p.M = d->num_heads; p.D = d->channels;
   p.L = d->num_levels; p.Lq = d->num_query; p.P = d->num_point;
+  p.value = value; p.shapes = shapes; p.lsi = lsi; p.loc = loc; p.aw = aw;
+}
+
+// Common tail of the forward entry points: chunk the queries for CTAs that serve `per_iter` of them per pass, then
+// `launch()` (0 or a return code) and count it.
+template <class Launch>
+static int forward_tail(const msda_dims* d, Params& p, int per_iter, Launch&& launch) {
+  p.qc = pick_chunk(d, per_iter, g_qc_fwd.load());
+  p.nchunk = (p.Lq + p.qc - 1) / p.qc;
+  if (int e = launch()) return e;
+  g_launches.fetch_add(1);
+  return 0;
+}
+
+// Where the scatter accumulates grad_value: grad_value itself for f32 / f64; for bf16 / f16 the fp32 scratch at the start of
+// the workspace, converted into grad_value afterwards.
+static void* backward_accum(int dtype, void* grad_value, void* workspace) {
+  return dtype == MSDA_BF16 || dtype == MSDA_F16 ? workspace : grad_value;
+}
+
+// The backward after its argument checks, shared by both entry points: chunk the queries, zero-fill the accumulator, let
+// `scatter(&launches)` accumulate into p.grad_value (0 or a return code; it sets `launches` if it issues more than one kernel),
+// convert a 16-bit result, count the launches. `vec`: the 4-channel lane layout (G = D / 4) applies; the fused entry points
+// (the ones that set p.ref) always meet it and the conditions of the packed 16-bit kernels.
+template <class Scatter>
+static int backward_body(const char* who, const msda_dims* dims, int dtype, Params& p, bool vec, void* grad_value,
+                         void* workspace, cudaStream_t s, Scatter&& scatter) {
+  const int G = p.D / 4;
+  p.qc = pick_chunk(dims, vec ? kWarps * (32 / G) : kWarps, g_qc_bwd.load());
+  p.nchunk = (p.Lq + p.qc - 1) / p.qc;
+  const size_t nvalue = (size_t)p.N * p.S * p.M * p.D;
+  const bool lowp = dtype == MSDA_BF16 || dtype == MSDA_F16;
+  // packed 16-bit reductions straight into grad_value (no fp32 scratch, no convert; see msda_bwd.cu red_add_16x4)
+  if (lowp && vec && g_bwd_packed16.load() == 2 && (G == 8 || G == 16) && ((p.L == 3 || p.L == 1) && p.P == 4) &&
+      aligned(grad_value, 8)) {
+    p.grad_value = grad_value;
+    cudaError_t e = cudaMemsetAsync(grad_value, 0, nvalue * elem_size(dtype), s);
+    if (e != cudaSuccess) return cuda_fail(e, "%s memset(grad_value)", who);
+    e = launch_backward_packed16(p, dtype, G, p.ref != nullptr, s);
+    if (e != cudaSuccess) return cuda_fail(e, "%s (packed 16-bit reductions) launch", who);
+    g_launches.fetch_add(1);
+    return 0;
+  }
+  p.grad_value = backward_accum(dtype, grad_value, workspace);
+  cudaError_t e = cudaMemsetAsync(p.grad_value, 0, nvalue * (lowp ? sizeof(float) : elem_size(dtype)), s);
+  if (e != cudaSuccess) return cuda_fail(e, "%s memset(grad_value)", who);
+  int launches = 1;
+  if (int rc = scatter(&launches)) return rc;
+  g_launches.fetch_add(launches);
+  if (lowp) {
+    e = launch_cvt_f32_bf16(reinterpret_cast<const float*>(p.grad_value), grad_value, nvalue, dtype, s);
+    if (e != cudaSuccess) return cuda_fail(e, "%s bf16 convert launch", who);
+    g_launches.fetch_add(1);
+  }
+  return 0;
 }
 
 // ---- debug: per-point index dump (same point_geom the kernels use) -----------------------------
@@ -350,9 +421,8 @@ int msda_forward_ex(const msda_dims* dims, int dtype, const void* value, const i
     return fail(MSDA_E_ALIGN, "msda_forward: pointer not aligned to its element size");
 
   Params p;
-  fill_params(p, dims);
-  p.value = value; p.shapes = spatial_shapes; p.lsi = level_start_index;
-  p.loc = sampling_loc; p.aw = attn_weight; p.out = out;
+  fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_loc, attn_weight);
+  p.out = out;
 
   int G = 0;
   bool vec = vec_supported(dtype, p.D, &G) && aligned(value, 16) && aligned(out, 16) &&
@@ -384,14 +454,9 @@ int msda_forward_ex(const msda_dims* dims, int dtype, const void* value, const i
       if (ew != cudaErrorNotSupported) return cuda_fail(ew, "msda_forward (32-byte lanes) launch");
     }
   }
-  const int per_iter = vec ? kWarps * (32 / G) : kWarps;
-  p.qc = pick_chunk(dims, per_iter, g_qc_fwd.load());
-  p.nchunk = (p.Lq + p.qc - 1) / p.qc;
-
-  const cudaError_t e = launch_forward(p, dtype, vec, G, g_minb_fwd.load(), (cudaStream_t)stream);
-  if (e != cudaSuccess) return cuda_fail(e, "msda_forward launch");
-  g_launches.fetch_add(1);
-  return 0;
+  return forward_tail(dims, p, vec ? kWarps * (32 / G) : kWarps, [&] {
+    return launched(launch_forward(p, dtype, vec, G, g_minb_fwd.load(), (cudaStream_t)stream), "msda_forward launch");
+  });
 }
 
 // fp32 accumulator of the 16-bit dtypes (first in the workspace), then the sort buffers of the slab-sorted backward
@@ -448,61 +513,26 @@ int msda_backward(const msda_dims* dims, int dtype, const void* value, const int
     return fail(MSDA_E_WORKSPACE, "msda_backward: workspace of %zu bytes (16-byte aligned) required, got %zu",
                 need, workspace ? workspace_bytes : (size_t)0);
 
-  cudaStream_t s = (cudaStream_t)stream;
   Params p;
-  fill_params(p, dims);
-  p.value = value; p.shapes = spatial_shapes; p.lsi = level_start_index;
-  p.loc = sampling_loc; p.aw = attn_weight; p.grad_out = grad_out;
-  p.grad_loc = grad_sampling_loc; p.grad_aw = grad_attn_weight;
+  fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_loc, attn_weight);
+  p.grad_out = grad_out; p.grad_loc = grad_sampling_loc; p.grad_aw = grad_attn_weight;
 
-  const size_t nvalue = (size_t)p.N * p.S * p.M * p.D;
-  const bool lowp = dtype == MSDA_BF16 || dtype == MSDA_F16;   // 16-bit I/O: fp32 accumulator in the workspace, converted once
-  void* accum = lowp ? workspace : grad_value;
-  const size_t accum_bytes = lowp ? nvalue * sizeof(float) : nvalue * es;
-  p.grad_value = accum;
-
-  // backward lane layout: 4 channels per lane for both dtypes (see VecB in msda_bwd.cu)
-  int G = p.D / 4;
-  bool vec = (dtype == MSDA_F32 || lowp) && p.D % 4 == 0 && G >= 2 && G <= 32 && (G & (G - 1)) == 0 &&
-             aligned(value, 16) && aligned(grad_out, 16) &&
-             aligned(accum, 16) && aligned(sampling_loc, 8) && aligned(grad_sampling_loc, 8);
-  const int per_iter = vec ? kWarps * (32 / G) : kWarps;
-  p.qc = pick_chunk(dims, per_iter, g_qc_bwd.load());
-  p.nchunk = (p.Lq + p.qc - 1) / p.qc;
-
-  // opt-in: packed 16-bit reductions straight into grad_value (no fp32 scratch, no convert; see msda_bwd.cu red_add_16x4)
-  if (lowp && vec && g_bwd_packed16.load() == 2 && (G == 8 || G == 16) && ((p.L == 3 || p.L == 1) && p.P == 4) && aligned(grad_value, 8)) {
-    p.grad_value = grad_value;
-    cudaError_t ep = cudaMemsetAsync(grad_value, 0, nvalue * es, s);
-    if (ep != cudaSuccess) return cuda_fail(ep, "msda_backward memset(grad_value)");
-    ep = launch_backward_packed16(p, dtype, G, false, s);
-    if (ep != cudaSuccess) return cuda_fail(ep, "msda_backward (packed 16-bit reductions) launch");
-    g_launches.fetch_add(1);
-    return 0;
-  }
-  cudaError_t e = cudaMemsetAsync(accum, 0, accum_bytes, s);
-  if (e != cudaSuccess) return cuda_fail(e, "msda_backward memset(grad_value)");
-  CellPlan cplan;
-  const size_t sorted_bytes = sorted_workspace_bytes(dims, dtype);
-  if (vec && sorted_bytes > 0) {
-    int n = 0;
-    e = launch_backward_sorted(p, dtype, reinterpret_cast<char*>(workspace) + accum_workspace_bytes(dims, dtype), sm_count(), &n, s);
-    if (e != cudaSuccess) return cuda_fail(e, "msda_backward (slab-sorted) launch");
-    g_launches.fetch_add(n - 1);
-  } else if (vec && plan_cell(dims, dtype, p, &cplan)) {
-    e = launch_backward_cell(p, cplan, dtype, s);
-    if (e != cudaSuccess) return cuda_fail(e, "msda_backward (cell-bucketed) launch");
-  } else {
-    e = launch_backward(p, dtype, vec, G, g_minb_bwd.load(), s);
-    if (e != cudaSuccess) return cuda_fail(e, "msda_backward launch");
-  }
-  g_launches.fetch_add(1);
-  if (lowp) {
-    e = launch_cvt_f32_bf16(reinterpret_cast<const float*>(accum), grad_value, nvalue, dtype, s);
-    if (e != cudaSuccess) return cuda_fail(e, "msda_backward bf16 convert launch");
-    g_launches.fetch_add(1);
-  }
-  return 0;
+  // backward lane layout: 4 channels per lane for every dtype (see VecB in msda_bwd.cu)
+  const int G = p.D / 4;
+  const bool vec = (dtype == MSDA_F32 || dtype == MSDA_BF16 || dtype == MSDA_F16) && p.D % 4 == 0 && G >= 2 && G <= 32 &&
+                   (G & (G - 1)) == 0 && aligned(value, 16) && aligned(grad_out, 16) && aligned(sampling_loc, 8) &&
+                   aligned(grad_sampling_loc, 8) && aligned(backward_accum(dtype, grad_value, workspace), 16);
+  const cudaStream_t s = (cudaStream_t)stream;
+  return backward_body("msda_backward", dims, dtype, p, vec, grad_value, workspace, s, [&](int* launches) {
+    CellPlan cplan;
+    if (vec && sorted_workspace_bytes(dims, dtype) > 0)
+      return launched(launch_backward_sorted(p, dtype, reinterpret_cast<char*>(workspace) + accum_workspace_bytes(dims, dtype),
+                                             sm_count(), launches, s),
+                      "msda_backward (slab-sorted) launch");
+    if (vec && plan_cell(dims, dtype, p, &cplan))
+      return launched(launch_backward_cell(p, cplan, dtype, s), "msda_backward (cell-bucketed) launch");
+    return launched(launch_backward(p, dtype, vec, G, g_minb_bwd.load(), s), "msda_backward launch");
+  });
 }
 
 static int fused_ref_params(Params& p, const msda_dims* d, const float* ref, int32_t ref_batch, int32_t ref_levels,
@@ -540,17 +570,12 @@ int msda_forward_fused(const msda_dims* dims, int dtype, const void* value, cons
       !aligned(spatial_shapes, 8) || !aligned(level_start_index, 8))
     return fail(MSDA_E_ALIGN, "msda_forward_fused: misaligned pointer");
   Params p;
-  fill_params(p, dims);
-  p.value = value; p.shapes = spatial_shapes; p.lsi = level_start_index;
-  p.loc = sampling_offsets; p.aw = attn_logits; p.out = out;
+  fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits);
+  p.out = out;
   if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, offsets_row_stride, logits_row_stride)) return e;
-  p.qc = pick_chunk(dims, kWarps * (32 / G), g_qc_fwd.load());
-  p.nchunk = (p.Lq + p.qc - 1) / p.qc;
-  const cudaError_t e = launch_forward_fused(p, dtype, G, (cudaStream_t)stream);
-  if (e == cudaErrorNotSupported) return fail(MSDA_E_UNSUPPORTED, "msda_forward_fused: no fused kernel for G=%d", G);
-  if (e != cudaSuccess) return cuda_fail(e, "msda_forward_fused launch");
-  g_launches.fetch_add(1);
-  return 0;
+  return forward_tail(dims, p, kWarps * (32 / G), [&] {
+    return fused_launched(launch_forward_fused(p, dtype, G, (cudaStream_t)stream), "msda_forward_fused", G);
+  });
 }
 
 int msda_backward_fused(const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
@@ -571,43 +596,17 @@ int msda_backward_fused(const msda_dims* dims, int dtype, const void* value, con
   const size_t need = accum_workspace_bytes(dims, dtype);
   if (need > 0 && (!workspace || workspace_bytes < need || !aligned(workspace, 16)))
     return fail(MSDA_E_WORKSPACE, "msda_backward_fused: workspace of %zu bytes (16-byte aligned) required", need);
-  cudaStream_t s = (cudaStream_t)stream;
   Params p;
-  fill_params(p, dims);
-  p.value = value; p.shapes = spatial_shapes; p.lsi = level_start_index;
-  p.loc = sampling_offsets; p.aw = attn_logits; p.grad_out = grad_out;
-  p.grad_loc = grad_sampling_offsets; p.grad_aw = grad_attn_logits;
+  fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits);
+  p.grad_out = grad_out; p.grad_loc = grad_sampling_offsets; p.grad_aw = grad_attn_logits;
   if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, offsets_row_stride, logits_row_stride)) return e;
-  const size_t nvalue = (size_t)p.N * p.S * p.M * p.D;
-  const bool lowp = dtype == MSDA_BF16 || dtype == MSDA_F16;   // 16-bit I/O: fp32 accumulator in the workspace, converted once
-  void* accum = lowp ? workspace : grad_value;
-  p.grad_value = accum;
-  if (!aligned(value, 16) || !aligned(grad_out, 16) || !aligned(accum, 16) || !aligned(sampling_offsets, 8) ||
-      !aligned(grad_sampling_offsets, 8))
+  if (!aligned(value, 16) || !aligned(grad_out, 16) || !aligned(backward_accum(dtype, grad_value, workspace), 16) ||
+      !aligned(sampling_offsets, 8) || !aligned(grad_sampling_offsets, 8))
     return fail(MSDA_E_ALIGN, "msda_backward_fused: misaligned pointer");
-  p.qc = pick_chunk(dims, kWarps * (32 / G), g_qc_bwd.load());
-  p.nchunk = (p.Lq + p.qc - 1) / p.qc;
-  if (lowp && g_bwd_packed16.load() == 2 && aligned(grad_value, 8)) {
-    p.grad_value = grad_value;
-    cudaError_t ep = cudaMemsetAsync(grad_value, 0, nvalue * elem_size(dtype), s);
-    if (ep != cudaSuccess) return cuda_fail(ep, "msda_backward_fused memset(grad_value)");
-    ep = launch_backward_packed16(p, dtype, G, true, s);
-    if (ep != cudaSuccess) return cuda_fail(ep, "msda_backward_fused (packed 16-bit reductions) launch");
-    g_launches.fetch_add(1);
-    return 0;
-  }
-  cudaError_t e = cudaMemsetAsync(accum, 0, nvalue * 4u, s);
-  if (e != cudaSuccess) return cuda_fail(e, "msda_backward_fused memset(grad_value)");
-  e = launch_backward_fused(p, dtype, G, s);
-  if (e == cudaErrorNotSupported) return fail(MSDA_E_UNSUPPORTED, "msda_backward_fused: no fused kernel for G=%d", G);
-  if (e != cudaSuccess) return cuda_fail(e, "msda_backward_fused launch");
-  g_launches.fetch_add(1);
-  if (lowp) {
-    e = launch_cvt_f32_bf16(reinterpret_cast<const float*>(accum), grad_value, nvalue, dtype, s);
-    if (e != cudaSuccess) return cuda_fail(e, "msda_backward_fused bf16 convert launch");
-    g_launches.fetch_add(1);
-  }
-  return 0;
+  const cudaStream_t s = (cudaStream_t)stream;
+  return backward_body("msda_backward_fused", dims, dtype, p, true, grad_value, workspace, s, [&](int*) {
+    return fused_launched(launch_backward_fused(p, dtype, G, s), "msda_backward_fused", G);
+  });
 }
 
 static size_t adapter_elem_size(int dtype) { return elem_size(dtype); }

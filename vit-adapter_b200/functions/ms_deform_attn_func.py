@@ -27,6 +27,21 @@ def set_amp_value_dtype(dtype):
     _AMP_VALUE_DTYPE = dtype
 
 
+def _amp_value(value):
+    """`value` in the dtype the kernels run on: the AMP value dtype under CUDA autocast, and fp16 up-cast to fp32 unless fp16
+    was asked for (the reference's behaviour for fp16 AMP: the core runs in fp32)."""
+    if torch.is_autocast_enabled('cuda') and value.is_cuda:
+        value = value.to(_AMP_VALUE_DTYPE)
+    if value.dtype == torch.float16 and _AMP_VALUE_DTYPE != torch.float16:
+        value = value.float()
+    return value
+
+
+def _grad_output(grad_output, value):
+    """grad_output contiguous and in value's dtype, as the backward kernels read it."""
+    return grad_output.to(value.dtype).contiguous()
+
+
 def _coord_dtype(value_dtype):
     return torch.float64 if value_dtype == torch.float64 else torch.float32
 
@@ -36,10 +51,7 @@ class MSDeformAttnFunction(Function):
     @staticmethod
     def forward(ctx, value, value_spatial_shapes, value_level_start_index,
                 sampling_locations, attention_weights, im2col_step):
-        if torch.is_autocast_enabled('cuda') and value.is_cuda:
-            value = value.to(_AMP_VALUE_DTYPE)
-        if value.dtype == torch.float16 and _AMP_VALUE_DTYPE != torch.float16:
-            value = value.float()   # the reference's behaviour for fp16 AMP: the core runs in fp32
+        value = _amp_value(value)
         cdt = _coord_dtype(value.dtype)
         # .to() is a no-op (same tensor) when the dtype already matches
         sampling_locations = sampling_locations.to(cdt)
@@ -55,11 +67,8 @@ class MSDeformAttnFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         value, shapes, level_start, loc, attn = ctx.saved_tensors
-        if grad_output.dtype != value.dtype:
-            grad_output = grad_output.to(value.dtype)
-        grad_output = grad_output.contiguous()
         grad_value, grad_loc, grad_attn = _cabi.backward(
-            value, shapes, level_start, loc, attn, grad_output, ctx.im2col_step)
+            value, shapes, level_start, loc, attn, _grad_output(grad_output, value), ctx.im2col_step)
         return grad_value, None, None, grad_loc, grad_attn, None
 
 
@@ -78,10 +87,7 @@ class MSDeformAttnFusedFunction(Function):
     @staticmethod
     def forward(ctx, value, value_spatial_shapes, value_level_start_index, reference_points, sampling_offsets,
                 attn_logits):
-        if torch.is_autocast_enabled('cuda') and value.is_cuda:
-            value = value.to(_AMP_VALUE_DTYPE)
-        if value.dtype == torch.float16 and _AMP_VALUE_DTYPE != torch.float16:
-            value = value.float()   # the reference's behaviour for fp16 AMP: the core runs in fp32
+        value = _amp_value(value)
         reference_points = reference_points.float().contiguous()
         sampling_offsets = sampling_offsets.float().contiguous()
         attn_logits = attn_logits.float().contiguous()
@@ -95,10 +101,8 @@ class MSDeformAttnFusedFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         value, shapes, level_start, ref, offsets, logits = ctx.saved_tensors
-        if grad_output.dtype != value.dtype:
-            grad_output = grad_output.to(value.dtype)
         grad_value, grad_off, grad_logits = _cabi.backward_fused(value, shapes, level_start, ref, offsets, logits,
-                                                                 grad_output.contiguous())
+                                                                 _grad_output(grad_output, value))
         return grad_value, None, None, None, grad_off, grad_logits
 
 
@@ -111,10 +115,7 @@ class MSDeformAttnMergedFunction(Function):
 
     @staticmethod
     def forward(ctx, value, value_spatial_shapes, value_level_start_index, reference_points, merged, n_levels, n_points):
-        if torch.is_autocast_enabled('cuda') and value.is_cuda:
-            value = value.to(_AMP_VALUE_DTYPE)
-        if value.dtype == torch.float16 and _AMP_VALUE_DTYPE != torch.float16:
-            value = value.float()   # the reference's behaviour for fp16 AMP: the core runs in fp32
+        value = _amp_value(value)
         reference_points = reference_points.float().contiguous()
         merged = merged.float().contiguous()
         ctx.lp = (int(n_levels), int(n_points))
@@ -127,8 +128,6 @@ class MSDeformAttnMergedFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         value, shapes, level_start, ref, merged = ctx.saved_tensors
-        if grad_output.dtype != value.dtype:
-            grad_output = grad_output.to(value.dtype)
         grad_value, grad_merged = _cabi.backward_fused_merged(value, shapes, level_start, ref, merged, *ctx.lp,
-                                                              grad_output.contiguous())
+                                                              _grad_output(grad_output, value))
         return grad_value, None, None, None, grad_merged, None, None
