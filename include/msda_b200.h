@@ -158,8 +158,11 @@ int msda_backward(const msda_dims* dims, int dtype,
  *                     [N*Lq, M*L*P*3] (`sampling_offsets` and `attention_weights` share the same input); the
  *                     gradients are written with the same strides, so they form the merged GEMM's output gradient.
  * The backward returns gradients w.r.t. the raw offsets and logits (softmax backward folded in).
- * Supported: dtype f32 / bf16, (L, P) in {(3,4), (1,4)}, D*sizeof(T) a multiple of 16 with 2..32 lanes;
- * anything else returns MSDA_E_UNSUPPORTED and the caller uses msda_forward / msda_backward. */
+ * Supported: dtype f32 / bf16 / f16, (L, P) in {(3,4), (1,4), (4,4)}, D = 32 or 64 (D*sizeof(T) a multiple of 16 with
+ * 2..32 lanes in the forward, D / 4 in {8, 16} in the backward); anything else returns MSDA_E_UNSUPPORTED and the
+ * caller uses msda_forward / msda_backward.
+ * msda_forward_fused / msda_backward_fused are msda_forward_fused_ref / msda_backward_fused_ref with ref_dim = 2 and
+ * grad_reference_points = NULL. */
 int msda_forward_fused(const msda_dims* dims, int dtype,
                        const void* value,
                        const int64_t* spatial_shapes,
@@ -185,6 +188,51 @@ int msda_backward_fused(const msda_dims* dims, int dtype,
                         float* grad_attn_logits,
                         void* workspace, size_t workspace_bytes,
                         void* stream);
+
+/* Fused entry points for every reference-point form the reference module accepts (ms_deform_attn.py:115-122):
+ *   ref_dim 2: reference_points [ref_batch, Lq, ref_levels, 2]  points (x, y):
+ *              sampling_location = reference_point + sampling_offset / (W_l, H_l)
+ *   ref_dim 4: reference_points [ref_batch, Lq, ref_levels, 4]  boxes (x, y, w, h), 16-byte aligned:
+ *              sampling_location = (x, y) + sampling_offset / P * (w, h) * 0.5
+ *              (torch's fp32 operations in torch's order: the locations are bit-identical to the unfused path)
+ * anything else returns MSDA_E_DIMS; a misaligned box returns MSDA_E_ALIGN.
+ * grad_reference_points: NULL = not wanted (the backward then launches exactly what msda_backward_fused launches), or
+ *   f32 [ref_batch, Lq, ref_levels, ref_dim], fully written by the call. The sum over heads, points (and levels /
+ *   batch where the reference points broadcast) uses no atomics: the result is bitwise reproducible. It needs the
+ *   larger workspace of msda_backward_fused_workspace_bytes(..., with_ref_grad = 1) and one more kernel launch. */
+int msda_forward_fused_ref(const msda_dims* dims, int dtype,
+                           const void* value,
+                           const int64_t* spatial_shapes,
+                           const int64_t* level_start_index,
+                           const float* reference_points, int32_t ref_batch, int32_t ref_levels, int32_t ref_dim,
+                           const float* sampling_offsets,
+                           const float* attn_logits,
+                           int64_t offsets_row_stride, int64_t logits_row_stride,
+                           void* out,
+                           void* stream);
+
+int msda_backward_fused_ref(const msda_dims* dims, int dtype,
+                            const void* value,
+                            const int64_t* spatial_shapes,
+                            const int64_t* level_start_index,
+                            const float* reference_points, int32_t ref_batch, int32_t ref_levels, int32_t ref_dim,
+                            const float* sampling_offsets,
+                            const float* attn_logits,
+                            int64_t offsets_row_stride, int64_t logits_row_stride,
+                            const void* grad_out,
+                            void* grad_value,
+                            float* grad_sampling_offsets,
+                            float* grad_attn_logits,
+                            float* grad_reference_points,
+                            void* workspace, size_t workspace_bytes,
+                            void* stream);
+
+/* Bytes of scratch the fused backward needs (16-byte aligned): the fp32 grad_value accumulator of the 16-bit dtypes
+ * (N*S*M*D floats; 0 for f32), then, when with_ref_grad != 0, the reference-point gradient partials at the next
+ * 16-byte boundary: N*Lq*M*ref_levels*ref_dim floats. 0 when dims is NULL, ref_dim is not 2 or 4, or the reference
+ * points do not broadcast (ref_batch not in {1, N}, ref_levels not in {1, L}). */
+size_t msda_backward_fused_workspace_bytes(const msda_dims* dims, int dtype, int32_t ref_batch, int32_t ref_levels,
+                                           int32_t ref_dim, int32_t with_ref_grad);
 
 /* ------------------------------------------------------------------------------------------------
  * Adapter ConvFFN depth-wise 3x3 convolution on the token layout (SURVEY.md §8(f) N3).

@@ -26,6 +26,7 @@ EXPORTS = (
     'msda_abi_version', 'msda_last_error', 'msda_check_im2col_step', 'msda_forward', 'msda_forward_ex',
     'msda_backward_workspace_bytes', 'msda_backward', 'msda_debug_point_index', 'msda_launch_count',
     'msda_set_tuning', 'msda_forward_fused', 'msda_backward_fused',
+    'msda_forward_fused_ref', 'msda_backward_fused_ref', 'msda_backward_fused_workspace_bytes',
     'adapter_dwconv_forward', 'adapter_dwconv_backward_input', 'adapter_dwconv_backward_weight',
     'adapter_dwconv_backward_weight_workspace_bytes',
     'adapter_layernorm_forward', 'adapter_layernorm_backward', 'adapter_layernorm_backward_workspace_bytes',
@@ -78,6 +79,16 @@ def load():
         lib.msda_backward_fused.restype = ctypes.c_int
         lib.msda_backward_fused.argtypes = [dp, ctypes.c_int, vp, i64p, i64p, vp, ctypes.c_int32, ctypes.c_int32, vp, vp,
                                             ctypes.c_int64, ctypes.c_int64, vp, vp, vp, vp, vp, ctypes.c_size_t, vp]
+        lib.msda_forward_fused_ref.restype = ctypes.c_int
+        lib.msda_forward_fused_ref.argtypes = [dp, ctypes.c_int, vp, i64p, i64p, vp, ctypes.c_int32, ctypes.c_int32,
+                                               ctypes.c_int32, vp, vp, ctypes.c_int64, ctypes.c_int64, vp, vp]
+        lib.msda_backward_fused_ref.restype = ctypes.c_int
+        lib.msda_backward_fused_ref.argtypes = [dp, ctypes.c_int, vp, i64p, i64p, vp, ctypes.c_int32, ctypes.c_int32,
+                                                ctypes.c_int32, vp, vp, ctypes.c_int64, ctypes.c_int64, vp, vp, vp, vp, vp, vp,
+                                                ctypes.c_size_t, vp]
+        lib.msda_backward_fused_workspace_bytes.restype = ctypes.c_size_t
+        lib.msda_backward_fused_workspace_bytes.argtypes = [dp, ctypes.c_int, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                                            ctypes.c_int32]
         i32 = ctypes.c_int32
         lib.adapter_dwconv_forward.restype = ctypes.c_int
         lib.adapter_dwconv_forward.argtypes = [ctypes.c_int, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
@@ -303,7 +314,7 @@ def fused_supported(value, n_levels, n_points):
     if not value.is_cuda or value.dtype not in (torch.float32, torch.bfloat16, torch.float16):
         return False
     D = value.shape[-1]
-    if not ((n_levels, n_points) in ((3, 4), (1, 4))) or D % 4 != 0 or (D // 4) not in (8, 16):
+    if not ((n_levels, n_points) in ((3, 4), (1, 4), (4, 4))) or D % 4 != 0 or (D // 4) not in (8, 16):
         return False
     cpl = 4 if value.dtype == torch.float32 else 8
     return D % cpl == 0 and (D // cpl) in (4, 8, 16)
@@ -316,13 +327,13 @@ def _check_fused_meta(spatial_shapes, level_start_index, reference_points, L):
     if tuple(spatial_shapes.shape) != (L, 2) or level_start_index.numel() != L:
         raise RuntimeError('fused MSDeformAttn: spatial_shapes must be [%d, 2] and level_start_index [%d], got %s and %s'
                            % (L, L, tuple(spatial_shapes.shape), tuple(level_start_index.shape)))
-    if reference_points.dim() != 4 or reference_points.shape[-1] != 2:
-        raise RuntimeError('fused MSDeformAttn: reference_points must be [Nr, Lq, Lr, 2], got %s' % (tuple(reference_points.shape),))
+    if reference_points.dim() != 4 or reference_points.shape[-1] not in (2, 4):
+        raise RuntimeError('fused MSDeformAttn: reference_points must be [Nr, Lq, Lr, 2|4], got %s' % (tuple(reference_points.shape),))
 
 
 def _fused_dims(value, reference_points, sampling_offsets, attn_logits):
-    if value.dim() != 4 or sampling_offsets.dim() != 6 or reference_points.dim() != 4 or reference_points.shape[-1] != 2:
-        raise RuntimeError('expected value [N,S,M,D], reference_points [Nr,Lq,Lr,2], sampling_offsets [N,Lq,M,L,P,2]')
+    if value.dim() != 4 or sampling_offsets.dim() != 6 or reference_points.dim() != 4 or reference_points.shape[-1] not in (2, 4):
+        raise RuntimeError('expected value [N,S,M,D], reference_points [Nr,Lq,Lr,2|4], sampling_offsets [N,Lq,M,L,P,2]')
     N, S, M, D = value.shape
     _, Lq, M2, L, P, _ = sampling_offsets.shape
     if M2 != M or attn_logits.numel() != N * Lq * M * L * P or reference_points.shape[1] != Lq:
@@ -332,37 +343,40 @@ def _fused_dims(value, reference_points, sampling_offsets, attn_logits):
     return MsdaDims(N, S, M, D, L, Lq, P), int(reference_points.shape[0]), int(reference_points.shape[2])
 
 
-def _forward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, offsets, logits, row_stride):
-    """out [N, Lq, M*D] of the fused entry. `row_stride`: floats between consecutive (b, q) rows of `offsets` and `logits`,
-    0 = dense. Runs under the caller's device guard."""
+def _forward_fused(dims, rb, rl, ref_dim, value, spatial_shapes, level_start_index, reference_points, offsets, logits,
+                   row_stride):
+    """out [N, Lq, M*D] of the fused entry. `ref_dim`: 2 (points) or 4 (boxes). `row_stride`: floats between consecutive
+    (b, q) rows of `offsets` and `logits`, 0 = dense. Runs under the caller's device guard."""
     _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
     out = torch.empty((dims.batch, dims.num_query, dims.num_heads * dims.channels), dtype=value.dtype, device=value.device)
-    rc = load().msda_forward_fused(ctypes.byref(dims), _DTYPES.get(value.dtype), value.data_ptr(), spatial_shapes.data_ptr(),
-                                   level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl, offsets.data_ptr(),
-                                   logits.data_ptr(), row_stride, row_stride, out.data_ptr(), _stream())
+    rc = load().msda_forward_fused_ref(ctypes.byref(dims), _DTYPES.get(value.dtype), value.data_ptr(), spatial_shapes.data_ptr(),
+                                       level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl, ref_dim,
+                                       offsets.data_ptr(), logits.data_ptr(), row_stride, row_stride, out.data_ptr(), _stream())
     if rc != 0:
-        _raise(rc, 'msda_forward_fused')
+        _raise(rc, 'msda_forward_fused_ref')
     return out
 
 
-def _backward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, offsets, logits, row_stride,
-                    grad_output, grad_offsets, grad_logits):
+def _backward_fused(dims, rb, rl, ref_dim, value, spatial_shapes, level_start_index, reference_points, offsets, logits,
+                    row_stride, grad_output, grad_offsets, grad_logits, grad_ref=None):
     """grad_value of the fused entry; writes the offset and logit gradients into `grad_offsets` / `grad_logits`, which have
-    the row stride of `offsets` / `logits`. Runs under the caller's device guard."""
+    the row stride of `offsets` / `logits`, and, when `grad_ref` (f32, the shape of `reference_points`) is given, the
+    reference-point gradient into it. Runs under the caller's device guard."""
     _check_fused_meta(spatial_shapes, level_start_index, reference_points, dims.num_levels)
     if grad_output.dtype != value.dtype:
         raise RuntimeError('grad_output dtype %s != value dtype %s' % (grad_output.dtype, value.dtype))
     lib = load()
     code = _DTYPES.get(value.dtype)
     grad_value = torch.empty_like(value)
-    ws_bytes = lib.msda_backward_workspace_bytes(ctypes.byref(dims), code)
+    ws_bytes = lib.msda_backward_fused_workspace_bytes(ctypes.byref(dims), code, rb, rl, ref_dim, grad_ref is not None)
     ws, ws_ptr = _workspace(ws_bytes, value.device)
-    rc = lib.msda_backward_fused(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
-                                 level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl, offsets.data_ptr(),
-                                 logits.data_ptr(), row_stride, row_stride, grad_output.data_ptr(), grad_value.data_ptr(),
-                                 grad_offsets.data_ptr(), grad_logits.data_ptr(), ws_ptr, ws_bytes, _stream())
+    rc = lib.msda_backward_fused_ref(ctypes.byref(dims), code, value.data_ptr(), spatial_shapes.data_ptr(),
+                                     level_start_index.data_ptr(), reference_points.data_ptr(), rb, rl, ref_dim,
+                                     offsets.data_ptr(), logits.data_ptr(), row_stride, row_stride, grad_output.data_ptr(),
+                                     grad_value.data_ptr(), grad_offsets.data_ptr(), grad_logits.data_ptr(),
+                                     grad_ref.data_ptr() if grad_ref is not None else None, ws_ptr, ws_bytes, _stream())
     if rc != 0:
-        _raise(rc, 'msda_backward_fused')
+        _raise(rc, 'msda_backward_fused_ref')
     return grad_value
 
 
@@ -372,26 +386,30 @@ def forward_fused(value, spatial_shapes, level_start_index, reference_points, sa
                       reference_points=reference_points, sampling_offsets=sampling_offsets, attn_logits=attn_logits)
     dims, rb, rl = _fused_dims(value, reference_points, sampling_offsets, attn_logits)
     with _on(dev):
-        return _forward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, sampling_offsets,
-                              attn_logits, 0)
+        return _forward_fused(dims, rb, rl, reference_points.shape[-1], value, spatial_shapes, level_start_index,
+                              reference_points, sampling_offsets, attn_logits, 0)
 
 
-def backward_fused(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits, grad_output):
-    """(grad_value, grad_sampling_offsets, grad_attn_logits) of the fused entry."""
+def backward_fused(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits, grad_output,
+                   ref_grad=False):
+    """(grad_value, grad_sampling_offsets, grad_attn_logits) of the fused entry, and grad_reference_points (f32, the shape of
+    `reference_points`) as a fourth element when `ref_grad`."""
     dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
                       reference_points=reference_points, sampling_offsets=sampling_offsets, attn_logits=attn_logits,
                       grad_output=grad_output)
     dims, rb, rl = _fused_dims(value, reference_points, sampling_offsets, attn_logits)
     with _on(dev):
         grad_off, grad_logits = torch.empty_like(sampling_offsets), torch.empty_like(attn_logits)
-        grad_value = _backward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points,
-                                     sampling_offsets, attn_logits, 0, grad_output, grad_off, grad_logits)
-    return grad_value, grad_off, grad_logits
+        grad_ref = torch.empty_like(reference_points) if ref_grad else None
+        grad_value = _backward_fused(dims, rb, rl, reference_points.shape[-1], value, spatial_shapes, level_start_index,
+                                     reference_points, sampling_offsets, attn_logits, 0, grad_output, grad_off, grad_logits,
+                                     grad_ref)
+    return (grad_value, grad_off, grad_logits) + ((grad_ref,) if ref_grad else ())
 
 
 def _merged_dims(value, reference_points, merged, n_levels, n_points):
-    if value.dim() != 4 or reference_points.dim() != 4 or reference_points.shape[-1] != 2:
-        raise RuntimeError('fused MSDeformAttn (merged): expected value [N,S,M,D] and reference_points [Nr,Lq,Lr,2], got %s and %s'
+    if value.dim() != 4 or reference_points.dim() != 4 or reference_points.shape[-1] not in (2, 4):
+        raise RuntimeError('fused MSDeformAttn (merged): expected value [N,S,M,D] and reference_points [Nr,Lq,Lr,2|4], got %s and %s'
                            % (tuple(value.shape), tuple(reference_points.shape)))
     N, S, M, D = value.shape
     Lq = reference_points.shape[1]
@@ -410,22 +428,25 @@ def forward_fused_merged(value, spatial_shapes, level_start_index, reference_poi
     dims, rb, rl, width = _merged_dims(value, reference_points, merged, n_levels, n_points)
     split = width // 3 * 2
     with _on(dev):
-        return _forward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points, merged[..., :split],
-                              merged[..., split:], width)
+        return _forward_fused(dims, rb, rl, reference_points.shape[-1], value, spatial_shapes, level_start_index,
+                              reference_points, merged[..., :split], merged[..., split:], width)
 
 
-def backward_fused_merged(value, spatial_shapes, level_start_index, reference_points, merged, n_levels, n_points, grad_output):
-    """(grad_value, grad_merged): grad_merged has the layout of `merged`, i.e. it is the merged GEMM's output gradient."""
+def backward_fused_merged(value, spatial_shapes, level_start_index, reference_points, merged, n_levels, n_points, grad_output,
+                          ref_grad=False):
+    """(grad_value, grad_merged): grad_merged has the layout of `merged`, i.e. it is the merged GEMM's output gradient;
+    grad_reference_points (f32, the shape of `reference_points`) follows as a third element when `ref_grad`."""
     dev = _check_cuda(value=value, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
                       reference_points=reference_points, merged=merged, grad_output=grad_output)
     dims, rb, rl, width = _merged_dims(value, reference_points, merged, n_levels, n_points)
     split = width // 3 * 2
     with _on(dev):
         grad_merged = torch.empty_like(merged)
-        grad_value = _backward_fused(dims, rb, rl, value, spatial_shapes, level_start_index, reference_points,
-                                     merged[..., :split], merged[..., split:], width, grad_output,
-                                     grad_merged[..., :split], grad_merged[..., split:])
-    return grad_value, grad_merged
+        grad_ref = torch.empty_like(reference_points) if ref_grad else None
+        grad_value = _backward_fused(dims, rb, rl, reference_points.shape[-1], value, spatial_shapes, level_start_index,
+                                     reference_points, merged[..., :split], merged[..., split:], width, grad_output,
+                                     grad_merged[..., :split], grad_merged[..., split:], grad_ref)
+    return (grad_value, grad_merged) + ((grad_ref,) if ref_grad else ())
 
 
 def dwconv_supported(x, weight, H, W):

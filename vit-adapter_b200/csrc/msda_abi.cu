@@ -19,6 +19,7 @@ cudaError_t launch_cvt_f32_bf16(const float* src, void* dst, size_t n, int dtype
 cudaError_t launch_backward_packed16(const Params& p, int dtype, int G, bool fused, cudaStream_t s);
 cudaError_t launch_forward_fused(const Params& p, int dtype, int G, cudaStream_t s);
 cudaError_t launch_backward_fused(const Params& p, int dtype, int G, cudaStream_t s);
+cudaError_t launch_ref_grad_reduce(const Params& p, int ref_batch, int ref_levels, float* grad_ref, cudaStream_t s);
 struct DwParams {
   const void* x;
   const void* w;
@@ -535,8 +536,29 @@ int msda_backward(const msda_dims* dims, int dtype, const void* value, const int
   });
 }
 
+// (L, P) of the fused kernels
+static bool fused_levels_points(const msda_dims* d) {
+  return (d->num_levels == 3 || d->num_levels == 1 || d->num_levels == 4) && d->num_point == 4;
+}
+
+static int check_ref_dim(int32_t ref_dim) {
+  if (ref_dim != 2 && ref_dim != 4) return fail(MSDA_E_DIMS, "fused entry: ref_dim=%d, expected 2 (points) or 4 (boxes)", ref_dim);
+  return 0;
+}
+
+static bool ref_broadcasts(const msda_dims* d, int32_t ref_batch, int32_t ref_levels) {
+  return (ref_batch == 1 || ref_batch == d->batch) && (ref_levels == 1 || ref_levels == d->num_levels);
+}
+
+static int check_ref_broadcast(const msda_dims* d, int32_t ref_batch, int32_t ref_levels, int32_t ref_dim) {
+  if (!ref_broadcasts(d, ref_batch, ref_levels))
+    return fail(MSDA_E_DIMS, "fused entry: reference_points [%d, Lq, %d, %d] does not broadcast to N=%d, L=%d", ref_batch,
+                ref_levels, ref_dim, d->batch, d->num_levels);
+  return 0;
+}
+
 static int fused_ref_params(Params& p, const msda_dims* d, const float* ref, int32_t ref_batch, int32_t ref_levels,
-                            int64_t off_rowstride, int64_t logit_rowstride) {
+                            int32_t ref_dim, int64_t off_rowstride, int64_t logit_rowstride) {
   const int64_t mlp = (int64_t)d->num_heads * d->num_levels * d->num_point;
   p.off_rowstride = off_rowstride > 0 ? off_rowstride : mlp * 2;
   p.logit_rowstride = logit_rowstride > 0 ? logit_rowstride : mlp;
@@ -544,38 +566,114 @@ static int fused_ref_params(Params& p, const msda_dims* d, const float* ref, int
     return fail(MSDA_E_DIMS, "fused entry: row strides (%lld, %lld) smaller than a row or odd", (long long)p.off_rowstride,
                 (long long)p.logit_rowstride);
   if (!ref) return fail(MSDA_E_NULL, "fused entry: reference_points is NULL");
-  if (!(ref_batch == 1 || ref_batch == d->batch) || !(ref_levels == 1 || ref_levels == d->num_levels))
-    return fail(MSDA_E_DIMS, "fused entry: reference_points [%d, Lq, %d, 2] does not broadcast to N=%d, L=%d", ref_batch,
-                ref_levels, d->batch, d->num_levels);
-  if (!aligned(ref, 8)) return fail(MSDA_E_ALIGN, "fused entry: reference_points not 8-byte aligned");
+  if (int e = check_ref_broadcast(d, ref_batch, ref_levels, ref_dim)) return e;
+  if (!aligned(ref, 4 * (size_t)ref_dim))  // one 8-byte (point) or 16-byte (box) load per reference point
+    return fail(MSDA_E_ALIGN, "fused entry: reference_points not %d-byte aligned", 4 * ref_dim);
   p.ref = ref;
-  p.ref_qstride = ref_levels * 2;
-  p.ref_lstride = ref_levels == 1 ? 0 : 2;
-  p.ref_bstride = ref_batch == 1 ? 0 : (long long)d->num_query * ref_levels * 2;
+  p.ref_dim = ref_dim;
+  p.ref_qstride = ref_levels * ref_dim;
+  p.ref_lstride = ref_levels == 1 ? 0 : ref_dim;
+  p.ref_bstride = ref_batch == 1 ? 0 : (long long)d->num_query * ref_levels * ref_dim;
   return 0;
+}
+
+// Backward scratch of the fused entry: the fp32 accumulator of the 16-bit dtypes, then (16-byte aligned) the
+// reference-point gradient partials [N, Lq, M, Lr, ref_dim] when that gradient is wanted.
+static size_t ref_partial_offset(const msda_dims* d, int dtype) { return (accum_workspace_bytes(d, dtype) + 15) & ~(size_t)15; }
+static size_t fused_workspace_bytes(const msda_dims* d, int dtype, int32_t ref_levels, int32_t ref_dim, bool with_ref_grad) {
+  if (!with_ref_grad) return accum_workspace_bytes(d, dtype);
+  return ref_partial_offset(d, dtype) +
+         (size_t)d->batch * d->num_query * d->num_heads * ref_levels * ref_dim * sizeof(float);
+}
+
+// The fused forward of both entry points (msda_forward_fused is the ref_dim = 2 case).
+static int forward_fused_body(const char* who, const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
+                              const int64_t* level_start_index, const float* reference_points, int32_t ref_batch,
+                              int32_t ref_levels, int32_t ref_dim, const float* sampling_offsets, const float* attn_logits,
+                              int64_t offsets_row_stride, int64_t logits_row_stride, void* out, void* stream) {
+  if (int e = check_dims(dims, dtype)) return e;
+  if (!value || !spatial_shapes || !level_start_index || !sampling_offsets || !attn_logits || !out)
+    return fail(MSDA_E_NULL, "%s: NULL tensor pointer", who);
+  int G = 0;
+  if (!vec_supported(dtype, dims->channels, &G) || !fused_levels_points(dims))
+    return fail(MSDA_E_UNSUPPORTED, "%s: no fused kernel for dtype=%d D=%d L=%d P=%d", who, dtype, dims->channels,
+                dims->num_levels, dims->num_point);
+  if (int e = check_ref_dim(ref_dim)) return e;
+  if (!aligned(value, 16) || !aligned(out, 16) || !aligned(sampling_offsets, 8) || !aligned(attn_logits, 4) ||
+      !aligned(spatial_shapes, 8) || !aligned(level_start_index, 8))
+    return fail(MSDA_E_ALIGN, "%s: misaligned pointer", who);
+  Params p;
+  fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits);
+  p.out = out;
+  if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, ref_dim, offsets_row_stride, logits_row_stride))
+    return e;
+  return forward_tail(dims, p, kWarps * (32 / G), [&] {
+    return fused_launched(launch_forward_fused(p, dtype, G, (cudaStream_t)stream), who, G);
+  });
 }
 
 int msda_forward_fused(const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
                        const int64_t* level_start_index, const float* reference_points, int32_t ref_batch,
                        int32_t ref_levels, const float* sampling_offsets, const float* attn_logits,
                        int64_t offsets_row_stride, int64_t logits_row_stride, void* out, void* stream) {
+  return forward_fused_body("msda_forward_fused", dims, dtype, value, spatial_shapes, level_start_index, reference_points,
+                            ref_batch, ref_levels, 2, sampling_offsets, attn_logits, offsets_row_stride, logits_row_stride,
+                            out, stream);
+}
+
+int msda_forward_fused_ref(const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
+                           const int64_t* level_start_index, const float* reference_points, int32_t ref_batch,
+                           int32_t ref_levels, int32_t ref_dim, const float* sampling_offsets, const float* attn_logits,
+                           int64_t offsets_row_stride, int64_t logits_row_stride, void* out, void* stream) {
+  return forward_fused_body("msda_forward_fused_ref", dims, dtype, value, spatial_shapes, level_start_index, reference_points,
+                            ref_batch, ref_levels, ref_dim, sampling_offsets, attn_logits, offsets_row_stride,
+                            logits_row_stride, out, stream);
+}
+
+// The fused backward of both entry points (msda_backward_fused is the ref_dim = 2, grad_reference_points = NULL case).
+static int backward_fused_body(const char* who, const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
+                               const int64_t* level_start_index, const float* reference_points, int32_t ref_batch,
+                               int32_t ref_levels, int32_t ref_dim, const float* sampling_offsets, const float* attn_logits,
+                               int64_t offsets_row_stride, int64_t logits_row_stride, const void* grad_out, void* grad_value,
+                               float* grad_sampling_offsets, float* grad_attn_logits, float* grad_reference_points,
+                               void* workspace, size_t workspace_bytes, void* stream) {
   if (int e = check_dims(dims, dtype)) return e;
-  if (!value || !spatial_shapes || !level_start_index || !sampling_offsets || !attn_logits || !out)
-    return fail(MSDA_E_NULL, "msda_forward_fused: NULL tensor pointer");
-  int G = 0;
-  if (!vec_supported(dtype, dims->channels, &G) || !((dims->num_levels == 3 || dims->num_levels == 1) && dims->num_point == 4))
-    return fail(MSDA_E_UNSUPPORTED, "msda_forward_fused: no fused kernel for dtype=%d D=%d L=%d P=%d", dtype, dims->channels,
+  if (!value || !spatial_shapes || !level_start_index || !sampling_offsets || !attn_logits || !grad_out || !grad_value ||
+      !grad_sampling_offsets || !grad_attn_logits)
+    return fail(MSDA_E_NULL, "%s: NULL tensor pointer", who);
+  const int G = dims->channels / 4;
+  if (!(dtype == MSDA_F32 || dtype == MSDA_BF16 || dtype == MSDA_F16) || dims->channels % 4 != 0 || !(G == 8 || G == 16) ||
+      !fused_levels_points(dims))
+    return fail(MSDA_E_UNSUPPORTED, "%s: no fused kernel for dtype=%d D=%d L=%d P=%d", who, dtype, dims->channels,
                 dims->num_levels, dims->num_point);
-  if (!aligned(value, 16) || !aligned(out, 16) || !aligned(sampling_offsets, 8) || !aligned(attn_logits, 4) ||
-      !aligned(spatial_shapes, 8) || !aligned(level_start_index, 8))
-    return fail(MSDA_E_ALIGN, "msda_forward_fused: misaligned pointer");
+  if (int e = check_ref_dim(ref_dim)) return e;
+  const bool ref_grad = grad_reference_points != nullptr;
+  // the size of the gradient's partials depends on ref_levels: check it before sizing the workspace
+  if (ref_grad)
+    if (int e = check_ref_broadcast(dims, ref_batch, ref_levels, ref_dim)) return e;
+  const size_t need = fused_workspace_bytes(dims, dtype, ref_levels, ref_dim, ref_grad);
+  if (need > 0 && (!workspace || workspace_bytes < need || !aligned(workspace, 16)))
+    return fail(MSDA_E_WORKSPACE, "%s: workspace of %zu bytes (16-byte aligned) required", who, need);
   Params p;
   fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits);
-  p.out = out;
-  if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, offsets_row_stride, logits_row_stride)) return e;
-  return forward_tail(dims, p, kWarps * (32 / G), [&] {
-    return fused_launched(launch_forward_fused(p, dtype, G, (cudaStream_t)stream), "msda_forward_fused", G);
-  });
+  p.grad_out = grad_out; p.grad_loc = grad_sampling_offsets; p.grad_aw = grad_attn_logits;
+  if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, ref_dim, offsets_row_stride, logits_row_stride))
+    return e;
+  if (!aligned(value, 16) || !aligned(grad_out, 16) || !aligned(backward_accum(dtype, grad_value, workspace), 16) ||
+      !aligned(sampling_offsets, 8) || !aligned(grad_sampling_offsets, 8) || (ref_grad && !aligned(grad_reference_points, 4)))
+    return fail(MSDA_E_ALIGN, "%s: misaligned pointer", who);
+  if (ref_grad) p.ref_partial = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + ref_partial_offset(dims, dtype));
+  const cudaStream_t s = (cudaStream_t)stream;
+  if (int rc = backward_body(who, dims, dtype, p, true, grad_value, workspace, s, [&](int*) {
+        return fused_launched(launch_backward_fused(p, dtype, G, s), who, G);
+      }))
+    return rc;
+  if (!ref_grad) return 0;
+  // every partial was written by the scatter kernel above: sum them into grad_reference_points in a fixed order
+  const cudaError_t e = launch_ref_grad_reduce(p, ref_batch, ref_levels, grad_reference_points, s);
+  if (e != cudaSuccess) return cuda_fail(e, "%s reference-point gradient launch", who);
+  g_launches.fetch_add(1);
+  return 0;
 }
 
 int msda_backward_fused(const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
@@ -584,29 +682,29 @@ int msda_backward_fused(const msda_dims* dims, int dtype, const void* value, con
                         int64_t offsets_row_stride, int64_t logits_row_stride,
                         const void* grad_out, void* grad_value, float* grad_sampling_offsets, float* grad_attn_logits,
                         void* workspace, size_t workspace_bytes, void* stream) {
-  if (int e = check_dims(dims, dtype)) return e;
-  if (!value || !spatial_shapes || !level_start_index || !sampling_offsets || !attn_logits || !grad_out || !grad_value ||
-      !grad_sampling_offsets || !grad_attn_logits)
-    return fail(MSDA_E_NULL, "msda_backward_fused: NULL tensor pointer");
-  const int G = dims->channels / 4;
-  if (!(dtype == MSDA_F32 || dtype == MSDA_BF16 || dtype == MSDA_F16) || dims->channels % 4 != 0 || !(G == 8 || G == 16) ||
-      !((dims->num_levels == 3 || dims->num_levels == 1) && dims->num_point == 4))
-    return fail(MSDA_E_UNSUPPORTED, "msda_backward_fused: no fused kernel for dtype=%d D=%d L=%d P=%d", dtype, dims->channels,
-                dims->num_levels, dims->num_point);
-  const size_t need = accum_workspace_bytes(dims, dtype);
-  if (need > 0 && (!workspace || workspace_bytes < need || !aligned(workspace, 16)))
-    return fail(MSDA_E_WORKSPACE, "msda_backward_fused: workspace of %zu bytes (16-byte aligned) required", need);
-  Params p;
-  fill_params(p, dims, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits);
-  p.grad_out = grad_out; p.grad_loc = grad_sampling_offsets; p.grad_aw = grad_attn_logits;
-  if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, offsets_row_stride, logits_row_stride)) return e;
-  if (!aligned(value, 16) || !aligned(grad_out, 16) || !aligned(backward_accum(dtype, grad_value, workspace), 16) ||
-      !aligned(sampling_offsets, 8) || !aligned(grad_sampling_offsets, 8))
-    return fail(MSDA_E_ALIGN, "msda_backward_fused: misaligned pointer");
-  const cudaStream_t s = (cudaStream_t)stream;
-  return backward_body("msda_backward_fused", dims, dtype, p, true, grad_value, workspace, s, [&](int*) {
-    return fused_launched(launch_backward_fused(p, dtype, G, s), "msda_backward_fused", G);
-  });
+  return backward_fused_body("msda_backward_fused", dims, dtype, value, spatial_shapes, level_start_index, reference_points,
+                             ref_batch, ref_levels, 2, sampling_offsets, attn_logits, offsets_row_stride, logits_row_stride,
+                             grad_out, grad_value, grad_sampling_offsets, grad_attn_logits, nullptr, workspace,
+                             workspace_bytes, stream);
+}
+
+int msda_backward_fused_ref(const msda_dims* dims, int dtype, const void* value, const int64_t* spatial_shapes,
+                            const int64_t* level_start_index, const float* reference_points, int32_t ref_batch,
+                            int32_t ref_levels, int32_t ref_dim, const float* sampling_offsets, const float* attn_logits,
+                            int64_t offsets_row_stride, int64_t logits_row_stride, const void* grad_out, void* grad_value,
+                            float* grad_sampling_offsets, float* grad_attn_logits, float* grad_reference_points,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  return backward_fused_body("msda_backward_fused_ref", dims, dtype, value, spatial_shapes, level_start_index,
+                             reference_points, ref_batch, ref_levels, ref_dim, sampling_offsets, attn_logits,
+                             offsets_row_stride, logits_row_stride, grad_out, grad_value, grad_sampling_offsets,
+                             grad_attn_logits, grad_reference_points, workspace, workspace_bytes, stream);
+}
+
+size_t msda_backward_fused_workspace_bytes(const msda_dims* dims, int dtype, int32_t ref_batch, int32_t ref_levels,
+                                           int32_t ref_dim, int32_t with_ref_grad) {
+  // the partials are per batch element whether or not the reference points broadcast over the batch
+  if (!dims || elem_size(dtype) == 0 || (ref_dim != 2 && ref_dim != 4) || !ref_broadcasts(dims, ref_batch, ref_levels)) return 0;
+  return fused_workspace_bytes(dims, dtype, ref_levels, ref_dim, with_ref_grad != 0);
 }
 
 static size_t adapter_elem_size(int dtype) { return elem_size(dtype); }

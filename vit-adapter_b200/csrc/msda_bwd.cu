@@ -131,10 +131,18 @@ __device__ __forceinline__ void group_transpose_sum(float (&v)[NV], int j) {
 // FUSED: `loc` / `aw` hold raw offsets / logits (see fused_resolve); grad_loc / grad_aw then receive the gradients
 // w.r.t. the raw offsets / logits (softmax backward and the 1/(W,H) scaling folded in).
 // PACK (16-bit T only): grad_value is T storage and the scatter uses packed 16-bit reductions (see red_add_16x4).
-template <typename T, int G, int LT, int PT, int MINB, bool FUSED = false, bool PACK = false>
+// RD (fused only): reference-point width, 2 = points (x, y), 4 = boxes (x, y, w, h).
+// RGRAD (fused only): also write the reference-point gradient of every (b,q,m) to p.ref_partial, reduced inside the group
+// over the P points of a level (and over the levels when the reference points broadcast over them); no atomics, so the
+// result is bitwise reproducible. msda_ref_grad_reduce_kernel sums the partials over the heads (and the batch).
+template <typename T, int G, int LT, int PT, int MINB, bool FUSED = false, bool PACK = false, int RD = 2, bool RGRAD = false>
 __global__ void __launch_bounds__(kThreads, MINB) msda_bwd_vec_kernel(const Params p) {
   static_assert(!FUSED || LT > 0, "the fused entry needs compile-time L, P");
   static_assert(!PACK || sizeof(T) == 2, "packed reductions are for the 16-bit value types");
+  static_assert((RD == 2 && !RGRAD) || (FUSED && (RD == 2 || RD == 4) && G % (PT > 0 ? PT : 1) == 0),
+                "box references and reference-point gradients are fused-entry features; a level's points share a round");
+  using RefV = RefVec<RD>;
+  constexpr float kInvP = 1.0f / (PT > 0 ? PT : 1);
   using V = VecB<T>;
   constexpr int kCpl = V::kCpl;
   constexpr int kGpw = 32 / G;
@@ -177,10 +185,11 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_bwd_vec_kernel(const Para
   // locations and attention weights are fetched before the current iteration is processed, so their HBM
   // latency is off the critical path.
   constexpr int kRounds = kStatic ? (LT * PT + G - 1) / G : 1;
-  float2 nxy[kRounds], nrf[kRounds];
+  float2 nxy[kRounds];
+  RefV nrf[kRounds];
   float na[kRounds];
   V ngo = V::zero();
-  auto fetch = [&](int qw_, float2 (&xy_)[kRounds], float (&a_)[kRounds], float2 (&rf_)[kRounds], V& go_) {
+  auto fetch = [&](int qw_, float2 (&xy_)[kRounds], float (&a_)[kRounds], RefV (&rf_)[kRounds], V& go_) {
     const int q_ = qw_ + grp;
     const bool act_ = q_ < bc.q_end;
     const int qq_ = act_ ? q_ : bc.q_begin;
@@ -190,7 +199,7 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_bwd_vec_kernel(const Para
     for (int r = 0; r < kRounds; ++r) {
       const int pi_ = r * G + j;
       xy_[r] = make_float2(0.f, 0.f);
-      rf_[r] = make_float2(0.f, 0.f);
+      rf_[r] = RefV{};
       a_[r] = 0.f;
       if (pi_ < LP && act_) {
         if (FUSED) {  // explicit row strides: offsets / logits may be column blocks of one merged GEMM output
@@ -202,8 +211,8 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_bwd_vec_kernel(const Para
           a_[r] = __ldg(aw + pair_ * LP + pi_);
         }
         if (FUSED)
-          rf_[r] = __ldg(reinterpret_cast<const float2*>(p.ref + (size_t)bc.b * p.ref_bstride + (size_t)qq_ * p.ref_qstride +
-                                                         (pi_ / (FUSED ? PT : 1)) * p.ref_lstride));
+          rf_[r] = __ldg(reinterpret_cast<const RefV*>(p.ref + (size_t)bc.b * p.ref_bstride + (size_t)qq_ * p.ref_qstride +
+                                                       (pi_ / (FUSED ? PT : 1)) * p.ref_lstride));
       }
     }
   };
@@ -217,14 +226,25 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_bwd_vec_kernel(const Para
     const float* __restrict__ aw_pair = aw + pair * LP;
 
     V go;
-    float2 cxy[kRounds], crf[kRounds];
+    float2 cxy[kRounds];
+    RefV crf[kRounds];
     float ca[kRounds];
     float ga_keep[kRounds];  // fused: d/d(attention weight) of this lane's points, kept for the softmax backward
     float dot_part = 0.f;    // fused: this lane's share of sum_p a_p * dL/da_p
+    float2 coff[RD == 4 && RGRAD ? kRounds : 1];  // boxes with RGRAD: the raw offsets (fused_resolve overwrites cxy)
+    float rsum[RGRAD ? RD : 1];  // RGRAD, levels broadcast: this (b,q,m)'s reference-point gradient summed over all points
+    if constexpr (RGRAD) {
+#pragma unroll
+      for (int c = 0; c < RD; ++c) rsum[c] = 0.f;
+    }
     if (kStatic) {
       go = ngo;
 #pragma unroll
       for (int r = 0; r < kRounds; ++r) { cxy[r] = nxy[r]; ca[r] = na[r]; crf[r] = nrf[r]; ga_keep[r] = 0.f; }
+      if constexpr (RD == 4 && RGRAD) {
+#pragma unroll
+        for (int r = 0; r < kRounds; ++r) coff[r] = cxy[r];
+      }
       if (qw + kWarps * kGpw < bc.q_end) fetch(qw + kWarps * kGpw, nxy, na, nrf, ngo);
       if constexpr (FUSED) fused_resolve<G, kRounds, (FUSED ? PT : 1)>(cxy, ca, crf, sH, sW, j, LP);
     } else {
@@ -331,16 +351,64 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_bwd_vec_kernel(const Para
         my_ga = part[0]; my_gw = part[1]; my_gh = part[2];
       }
       if constexpr (FUSED) {
-        // d loc / d offset = 1 / (W, H): the (W, H) factors of grad_sampling_loc cancel
-        if (mine) {
-          const size_t row = (size_t)bc.b * p.Lq + q;
-          *reinterpret_cast<float2*>(gloc + row * p.off_rowstride + (size_t)bc.m * LP * 2 + 2 * pi) = make_float2(my_gw * a, my_gh * a);
+        // dL/dloc exactly as the plain kernel writes grad_sampling_loc (boxes and reference-point gradients need it)
+        const float gx = fW * my_gw * a, gy = fH * my_gh * a;
+        if constexpr (RD == 2) {
+          // d loc / d offset = 1 / (W, H): the (W, H) factors of grad_sampling_loc cancel
+          if (mine) {
+            const size_t row = (size_t)bc.b * p.Lq + q;
+            *reinterpret_cast<float2*>(gloc + row * p.off_rowstride + (size_t)bc.m * LP * 2 + 2 * pi) = make_float2(my_gw * a, my_gh * a);
+          }
+        } else {
+          // boxes: d loc / d offset = ref_wh * 0.5 / P, applied in the order torch's autograd applies it
+          if (mine) {
+            const size_t row = (size_t)bc.b * p.Lq + q;
+            const RefV rf = crf[r0 / G];
+            *reinterpret_cast<float2*>(gloc + row * p.off_rowstride + (size_t)bc.m * LP * 2 + 2 * pi) =
+                make_float2(__fmul_rn(__fmul_rn(__fmul_rn(gx, 0.5f), rf.z), kInvP), __fmul_rn(__fmul_rn(__fmul_rn(gy, 0.5f), rf.w), kInvP));
+          }
+        }
+        if constexpr (RGRAD) {
+          // d ref_xy = dL/dloc; boxes: d ref_wh = (dL/dloc * 0.5) * (offset / P)
+          float gr[RD];
+          gr[0] = mine ? gx : 0.f;
+          gr[1] = mine ? gy : 0.f;
+          if constexpr (RD == 4) {
+            gr[2] = mine ? __fmul_rn(__fmul_rn(gx, 0.5f), __fmul_rn(coff[r0 / G].x, kInvP)) : 0.f;
+            gr[3] = mine ? __fmul_rn(__fmul_rn(gy, 0.5f), __fmul_rn(coff[r0 / G].y, kInvP)) : 0.f;
+          }
+          // the PT points of a level are PT aligned consecutive lanes of this round: sum them
+#pragma unroll
+          for (int s = 1; s < PT; s <<= 1)
+#pragma unroll
+            for (int c = 0; c < RD; ++c) gr[c] += __shfl_xor_sync(0xffffffffu, gr[c], s, G);
+          if (p.ref_lstride != 0) {  // one reference point per level: that level's partial is complete
+            if (mine && j % PT == 0) {
+              float* dst = p.ref_partial + ((((size_t)bc.b * p.Lq + q) * p.M + bc.m) * LT + pi / PT) * RD;
+              if constexpr (RD == 4) *reinterpret_cast<float4*>(dst) = make_float4(gr[0], gr[1], gr[2], gr[3]);
+              else *reinterpret_cast<float2*>(dst) = make_float2(gr[0], gr[1]);
+            }
+          } else {  // one reference point for all levels: sum the levels of this round, then the rounds
+#pragma unroll
+            for (int s = PT; s < G; s <<= 1)
+#pragma unroll
+              for (int c = 0; c < RD; ++c) gr[c] += __shfl_xor_sync(0xffffffffu, gr[c], s, G);
+#pragma unroll
+            for (int c = 0; c < RD; ++c) rsum[c] += gr[c];
+          }
         }
         ga_keep[r0 / G] = mine ? my_ga : 0.f;
         dot_part = fmaf(a, ga_keep[r0 / G], dot_part);
       } else if (mine) {
         gaw[pair * LP + pi] = my_ga;
         reinterpret_cast<float2*>(gloc)[pair * LP + pi] = make_float2(fW * my_gw * a, fH * my_gh * a);
+      }
+    }
+    if constexpr (RGRAD) {
+      if (p.ref_lstride == 0 && active && j == 0) {
+        float* dst = p.ref_partial + (((size_t)bc.b * p.Lq + q) * p.M + bc.m) * RD;
+        if constexpr (RD == 4) *reinterpret_cast<float4*>(dst) = make_float4(rsum[0], rsum[1], rsum[2], rsum[3]);
+        else *reinterpret_cast<float2*>(dst) = make_float2(rsum[0], rsum[1]);
       }
     }
     if constexpr (FUSED) {
@@ -463,12 +531,26 @@ static cudaError_t launch_vec_g(const Params& p, int minb, dim3 grid, cudaStream
   }
 }
 
+// The fused kernel for the call's reference width (p.ref_dim) and whether it writes reference-point gradient partials
+// (p.ref_partial): f(std::integral_constant<int, RD>, std::bool_constant<RGRAD>).
+template <class F>
+static cudaError_t with_ref_variant(const Params& p, F&& f) {
+  if (p.ref_dim == 4)
+    return p.ref_partial ? f(std::integral_constant<int, 4>{}, std::true_type{}) : f(std::integral_constant<int, 4>{}, std::false_type{});
+  return p.ref_partial ? f(std::integral_constant<int, 2>{}, std::true_type{}) : f(std::integral_constant<int, 2>{}, std::false_type{});
+}
+
 template <typename T, int G>
 static cudaError_t launch_fused_g(const Params& p, dim3 grid, cudaStream_t s) {
-  if (p.L == 3 && p.P == 4) msda_bwd_vec_kernel<T, G, 3, 4, 3, true><<<grid, kThreads, 0, s>>>(p);
-  else if (p.L == 1 && p.P == 4) msda_bwd_vec_kernel<T, G, 1, 4, 3, true><<<grid, kThreads, 0, s>>>(p);
-  else return cudaErrorNotSupported;
-  return cudaGetLastError();
+  return with_ref_variant(p, [&](auto rd, auto rg) {
+    constexpr int RD = decltype(rd)::value;
+    constexpr bool RG = decltype(rg)::value;
+    if (p.L == 3 && p.P == 4) msda_bwd_vec_kernel<T, G, 3, 4, 3, true, false, RD, RG><<<grid, kThreads, 0, s>>>(p);
+    else if (p.L == 1 && p.P == 4) msda_bwd_vec_kernel<T, G, 1, 4, 3, true, false, RD, RG><<<grid, kThreads, 0, s>>>(p);
+    else if (p.L == 4 && p.P == 4) msda_bwd_vec_kernel<T, G, 4, 4, 3, true, false, RD, RG><<<grid, kThreads, 0, s>>>(p);
+    else return cudaErrorNotSupported;
+    return cudaGetLastError();
+  });
 }
 
 template <typename T>
@@ -497,8 +579,13 @@ static cudaError_t launch_packed_g(const Params& p, bool fused, dim3 grid, cudaS
     const bool l3 = p.L == 3 && p.P == 4, l1 = p.L == 1 && p.P == 4;
     if (!l3 && !l1) return cudaErrorNotSupported;
     if (fused) {
-      if (l3) msda_bwd_vec_kernel<T, G, 3, 4, 3, true, true><<<grid, kThreads, 0, s>>>(p);
-      else msda_bwd_vec_kernel<T, G, 1, 4, 3, true, true><<<grid, kThreads, 0, s>>>(p);
+      return with_ref_variant(p, [&](auto rd, auto rg) {
+        constexpr int RD = decltype(rd)::value;
+        constexpr bool RG = decltype(rg)::value;
+        if (l3) msda_bwd_vec_kernel<T, G, 3, 4, 3, true, true, RD, RG><<<grid, kThreads, 0, s>>>(p);
+        else msda_bwd_vec_kernel<T, G, 1, 4, 3, true, true, RD, RG><<<grid, kThreads, 0, s>>>(p);
+        return cudaGetLastError();
+      });
     } else {
       if (l3) msda_bwd_vec_kernel<T, G, 3, 4, 3, false, true><<<grid, kThreads, 0, s>>>(p);
       else msda_bwd_vec_kernel<T, G, 1, 4, 3, false, true><<<grid, kThreads, 0, s>>>(p);
@@ -597,6 +684,35 @@ cudaError_t launch_backward_packed16(const Params& p, int dtype, int G, bool fus
 
 cudaError_t launch_cvt_f32_bf16(const float* src, void* dst, size_t n, int dtype, cudaStream_t s) {
   return dtype == MSDA_F16 ? bwd_cvt_f16(src, dst, n, s) : bwd_cvt_bf16(src, dst, n, s);
+}
+
+// grad_reference_points [Nr, Lq, Lr, RD] from the partials [N, Lq, M, Lr, RD] of the RGRAD fused backward: one thread per
+// output float sums over the heads (and over the batch when Nr == 1), always in the order b, then m.
+__global__ void __launch_bounds__(kThreads) msda_ref_grad_reduce_kernel(const float* __restrict__ partial, float* __restrict__ out,
+                                                                        int N, int Lq, int M, int Nr, int Lr, int RD) {
+  const size_t per_q = (size_t)Lr * RD;
+  const size_t total = (size_t)Nr * Lq * per_q;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const size_t lc = i % per_q;
+    const size_t q = (i / per_q) % Lq;
+    const int b0 = (int)(i / (per_q * Lq));
+    const int b1 = Nr == 1 ? N : b0 + 1;
+    float acc = 0.f;
+    for (int b = b0; b < b1; ++b) {
+      const float* src = partial + (((size_t)b * Lq + q) * M) * per_q + lc;
+      for (int m = 0; m < M; ++m) acc += src[(size_t)m * per_q];
+    }
+    out[i] = acc;
+  }
+}
+
+cudaError_t launch_ref_grad_reduce(const Params& p, int ref_batch, int ref_levels, float* grad_ref, cudaStream_t s) {
+  const size_t total = (size_t)ref_batch * p.Lq * ref_levels * p.ref_dim;
+  size_t blocks = (total + kThreads - 1) / kThreads;
+  if (blocks > 148u * 16u) blocks = 148u * 16u;
+  msda_ref_grad_reduce_kernel<<<(unsigned)blocks, kThreads, 0, s>>>(p.ref_partial, grad_ref, p.N, p.Lq, p.M, ref_batch, ref_levels,
+                                                                   p.ref_dim);
+  return cudaGetLastError();
 }
 #endif  // MSDA_TU
 

@@ -14,6 +14,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <type_traits>
 
 #include "../../include/msda_b200.h"
 
@@ -54,12 +55,14 @@ struct Params {
   int nchunk;              // ceil(Lq / qc)
   // fused entry points only: `loc` holds RAW sampling offsets, `aw` RAW attention logits, and the
   // locations / softmax are formed in registers from the reference points below
-  const float* ref;        // reference points [Nr, Lq, Lr, 2]
+  const float* ref;        // reference points [Nr, Lq, Lr, RD], RD = ref_dim
   long long ref_bstride;   // floats between batches (0 when Nr == 1: broadcast)
-  int ref_qstride;         // floats between queries (= Lr * 2)
+  int ref_qstride;         // floats between queries (= Lr * RD)
   int ref_lstride;         // floats between levels  (0 when Lr == 1: broadcast)
   long long off_rowstride;   // floats between the offsets of consecutive (b,q) rows (dense: M*L*P*2); same for their gradient
   long long logit_rowstride; // floats between the logits  of consecutive (b,q) rows (dense: M*L*P);   same for their gradient
+  int ref_dim;             // 2: points (x, y); 4: boxes (x, y, w, h)
+  float* ref_partial;      // fused bwd: NULL, or the per-(b, q, m, lr) reference-point gradient partials [N, Lq, M, Lr, RD]
 };
 
 // Host-made plan for the shared-memory forward (msda_fwd_smem.cu): which levels' [H*W, D] maps of one
@@ -243,16 +246,23 @@ struct Vec<__half> {
   }
 };
 
+// Reference point of one level as the fused kernels hold it: (x, y) or, for boxes, (x, y, w, h) in one 16-byte load.
+template <int RD>
+using RefVec = std::conditional_t<RD == 4, float4, float2>;
+
 // Fused module arithmetic (reference: detection/ops/modules/ms_deform_attn.py:108-119), done in registers:
 //   attention_weights = softmax(logits over the L*P points of one (b,q,m))
-//   sampling_location = reference_point + sampling_offset / (W_l, H_l)
+//   sampling_location = reference_point + sampling_offset / (W_l, H_l)                 (RD = 2)
+//   sampling_location = ref_xy + sampling_offset / P * ref_wh * 0.5                    (RD = 4, boxes)
 // Lane j of a G-lane group holds points j, j+G, ... (R rounds): xy[r] = raw offset, a[r] = raw logit,
 // rf[r] = reference point of that point's level. On return xy[r] = location, a[r] = softmax weight.
 // The max / sum over the L*P points are warp-shuffle reductions inside the group (every lane of the warp
-// must call this). Division and addition are the same fp32 operations torch performs, so the locations —
-// and therefore the corner indices — are bit-identical to the unfused path.
-template <int G, int R, int PT>
-__device__ __forceinline__ void fused_resolve(float2 (&xy)[R], float (&a)[R], const float2 (&rf)[R],
+// must call this). The location arithmetic is the fp32 operations torch performs, in its order and with its
+// roundings (a true division by the Python scalar P is torch's multiply by the reciprocal; the _rn intrinsics
+// keep nvcc from contracting into an FMA), so the locations — and therefore the corner indices — are
+// bit-identical to the unfused path.
+template <int G, int R, int PT, typename RefV>
+__device__ __forceinline__ void fused_resolve(float2 (&xy)[R], float (&a)[R], const RefV (&rf)[R],
                                               const int* sH, const int* sW, int j, int LP) {
   float m = -INFINITY;
 #pragma unroll
@@ -273,9 +283,15 @@ __device__ __forceinline__ void fused_resolve(float2 (&xy)[R], float (&a)[R], co
     a[r] = __fdiv_rn(a[r], sum);
     const int pi = r * G + j;
     if (pi < LP) {
-      const int l = pi / PT;
-      xy[r].x = rf[r].x + __fdiv_rn(xy[r].x, (float)sW[l]);
-      xy[r].y = rf[r].y + __fdiv_rn(xy[r].y, (float)sH[l]);
+      if constexpr (sizeof(RefV) == 16) {
+        constexpr float kInvP = 1.0f / PT;
+        xy[r].x = __fadd_rn(rf[r].x, __fmul_rn(__fmul_rn(__fmul_rn(xy[r].x, kInvP), rf[r].z), 0.5f));
+        xy[r].y = __fadd_rn(rf[r].y, __fmul_rn(__fmul_rn(__fmul_rn(xy[r].y, kInvP), rf[r].w), 0.5f));
+      } else {
+        const int l = pi / PT;
+        xy[r].x = rf[r].x + __fdiv_rn(xy[r].x, (float)sW[l]);
+        xy[r].y = rf[r].y + __fdiv_rn(xy[r].y, (float)sH[l]);
+      }
     }
   }
 }

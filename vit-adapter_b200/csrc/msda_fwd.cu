@@ -24,9 +24,12 @@ namespace msda {
 // LT/PT = compile-time levels / points (0,0 = runtime), MINB = min resident CTAs per SM.
 // ---------------------------------------------------------------------------------------------
 // FUSED: `loc` / `aw` hold raw offsets / logits; locations and the softmax are formed in registers (static L,P only).
-template <typename T, int G, int LT, int PT, int MINB, int LB = 16, bool FUSED = false>
+// RD (fused only): reference-point width, 2 = points (x, y), 4 = boxes (x, y, w, h).
+template <typename T, int G, int LT, int PT, int MINB, int LB = 16, bool FUSED = false, int RD = 2>
 __global__ void __launch_bounds__(kThreads, MINB) msda_fwd_vec_kernel(const Params p) {
   static_assert(!FUSED || LT > 0, "the fused entry needs compile-time L, P");
+  static_assert(RD == 2 || (FUSED && RD == 4), "box references are a fused-entry input");
+  using RefV = RefVec<RD>;
   using V = LaneVec<T, LB>;  // LB = bytes per lane: 16 (LDG.128) or 32 (LDG.256, fp32 only)
   constexpr int kCpl = V::kCpl;
   constexpr int kGpw = 32 / G;  // (b,q,m) groups per warp
@@ -71,9 +74,10 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_fwd_vec_kernel(const Para
   // latency (~800 cycles) would sit at the head of every iteration's dependency chain. The static
   // variants fetch the NEXT iteration's locations and weights before working on the current one.
   constexpr int kRounds = kStatic ? (LT * PT + G - 1) / G : 1;
-  float2 nxy[kRounds], nrf[kRounds];
+  float2 nxy[kRounds];
+  RefV nrf[kRounds];
   float na[kRounds];
-  auto fetch = [&](int qw_, float2 (&xy_)[kRounds], float (&a_)[kRounds], float2 (&rf_)[kRounds]) {
+  auto fetch = [&](int qw_, float2 (&xy_)[kRounds], float (&a_)[kRounds], RefV (&rf_)[kRounds]) {
     const int q_ = qw_ + grp;
     const bool act_ = q_ < bc.q_end;
     const int qq_ = act_ ? q_ : bc.q_begin;
@@ -82,7 +86,7 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_fwd_vec_kernel(const Para
     for (int r = 0; r < kRounds; ++r) {
       const int pi_ = r * G + j;
       xy_[r] = make_float2(0.f, 0.f);
-      rf_[r] = make_float2(0.f, 0.f);
+      rf_[r] = RefV{};
       a_[r] = 0.f;
       if (pi_ < LP && act_) {
         if (FUSED) {  // raw offsets / logits may be two column blocks of ONE merged GEMM output: explicit row strides
@@ -94,8 +98,8 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_fwd_vec_kernel(const Para
           a_[r] = __ldg(aw + pair_ * LP + pi_);
         }
         if (FUSED)
-          rf_[r] = __ldg(reinterpret_cast<const float2*>(p.ref + (size_t)bc.b * p.ref_bstride + (size_t)qq_ * p.ref_qstride +
-                                                         (pi_ / (FUSED ? PT : 1)) * p.ref_lstride));
+          rf_[r] = __ldg(reinterpret_cast<const RefV*>(p.ref + (size_t)bc.b * p.ref_bstride + (size_t)qq_ * p.ref_qstride +
+                                                       (pi_ / (FUSED ? PT : 1)) * p.ref_lstride));
       }
     }
   };
@@ -108,7 +112,8 @@ __global__ void __launch_bounds__(kThreads, MINB) msda_fwd_vec_kernel(const Para
     const float* __restrict__ loc_pair = loc + pair * LP * 2;
     const float* __restrict__ aw_pair = aw + pair * LP;
 
-    float2 cxy[kRounds], crf[kRounds];
+    float2 cxy[kRounds];
+    RefV crf[kRounds];
     float ca[kRounds];
     if (kStatic) {
 #pragma unroll
@@ -255,13 +260,18 @@ static cudaError_t launch_vec_g(const Params& p, int minb, dim3 grid, cudaStream
 #define MSDA_TU 0
 #endif
 
-// fused entry (raw offsets + logits + reference points): static (L,P) in {(3,4),(1,4)} only
-template <typename T, int G>
-static cudaError_t launch_fused_g(const Params& p, dim3 grid, cudaStream_t s) {
-  if (p.L == 3 && p.P == 4) msda_fwd_vec_kernel<T, G, 3, 4, 4, 16, true><<<grid, kThreads, 0, s>>>(p);
-  else if (p.L == 1 && p.P == 4) msda_fwd_vec_kernel<T, G, 1, 4, 4, 16, true><<<grid, kThreads, 0, s>>>(p);
+// fused entry (raw offsets + logits + reference points): static (L,P) in {(3,4),(1,4),(4,4)} only, points or boxes
+template <typename T, int G, int RD>
+static cudaError_t launch_fused_gr(const Params& p, dim3 grid, cudaStream_t s) {
+  if (p.L == 3 && p.P == 4) msda_fwd_vec_kernel<T, G, 3, 4, 4, 16, true, RD><<<grid, kThreads, 0, s>>>(p);
+  else if (p.L == 1 && p.P == 4) msda_fwd_vec_kernel<T, G, 1, 4, 4, 16, true, RD><<<grid, kThreads, 0, s>>>(p);
+  else if (p.L == 4 && p.P == 4) msda_fwd_vec_kernel<T, G, 4, 4, 4, 16, true, RD><<<grid, kThreads, 0, s>>>(p);
   else return cudaErrorNotSupported;
   return cudaGetLastError();
+}
+template <typename T, int G>
+static cudaError_t launch_fused_g(const Params& p, dim3 grid, cudaStream_t s) {
+  return p.ref_dim == 4 ? launch_fused_gr<T, G, 4>(p, grid, s) : launch_fused_gr<T, G, 2>(p, grid, s);
 }
 
 template <typename T>

@@ -42,6 +42,15 @@ def _grad_output(grad_output, value):
     return grad_output.to(value.dtype).contiguous()
 
 
+def _fused_ref(reference_points):
+    """reference_points as the fused kernels read them: fp32, contiguous, and aligned to one point (8 bytes) or box (16
+    bytes) - a view with an odd storage offset is copied."""
+    ref = reference_points.float().contiguous()
+    if ref.data_ptr() % (4 * ref.shape[-1]) != 0:
+        ref = ref.clone()
+    return ref
+
+
 def _coord_dtype(value_dtype):
     return torch.float64 if value_dtype == torch.float64 else torch.float32
 
@@ -79,16 +88,18 @@ class MSDeformAttnFusedFunction(Function):
         apply(value, spatial_shapes, level_start_index, reference_points, sampling_offsets, attn_logits)
 
     with RAW `sampling_offsets` [N,Lq,M,L,P,2] and RAW pre-softmax `attn_logits` [N,Lq,M,L*P]; the kernel forms
-    softmax(attn_logits) and reference_point + offset / (W_l, H_l) in registers, so neither tensor is written
-    to HBM, and the backward returns gradients w.r.t. the raw offsets / logits. `reference_points` is
-    [1|N, Lq, 1|L, 2] (no gradient, as in the adapter where it is a constant grid).
+    softmax(attn_logits) and the sampling locations in registers, so neither tensor is written to HBM, and the
+    backward returns gradients w.r.t. the raw offsets / logits. `reference_points` is [1|N, Lq, 1|L, 2] (points:
+    reference_point + offset / (W_l, H_l)) or [1|N, Lq, 1|L, 4] (boxes: xy + offset / P * wh * 0.5). Its gradient is
+    computed exactly when it requires one (Deformable-DETR style decoders); otherwise, as for the adapter's constant
+    grid, the backward launches no extra kernel.
     Same AMP policy as MSDeformAttnFunction. Use `_cabi.fused_supported` to check for a kernel."""
 
     @staticmethod
     def forward(ctx, value, value_spatial_shapes, value_level_start_index, reference_points, sampling_offsets,
                 attn_logits):
         value = _amp_value(value)
-        reference_points = reference_points.float().contiguous()
+        reference_points = _fused_ref(reference_points)
         sampling_offsets = sampling_offsets.float().contiguous()
         attn_logits = attn_logits.float().contiguous()
         output = _cabi.forward_fused(value, value_spatial_shapes, value_level_start_index, reference_points,
@@ -101,9 +112,11 @@ class MSDeformAttnFusedFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         value, shapes, level_start, ref, offsets, logits = ctx.saved_tensors
-        grad_value, grad_off, grad_logits = _cabi.backward_fused(value, shapes, level_start, ref, offsets, logits,
-                                                                 _grad_output(grad_output, value))
-        return grad_value, None, None, None, grad_off, grad_logits
+        want_ref = ctx.needs_input_grad[3]
+        grads = _cabi.backward_fused(value, shapes, level_start, ref, offsets, logits, _grad_output(grad_output, value),
+                                     ref_grad=want_ref)
+        grad_value, grad_off, grad_logits = grads[:3]
+        return grad_value, None, None, grads[3] if want_ref else None, grad_off, grad_logits
 
 
 class MSDeformAttnMergedFunction(Function):
@@ -111,12 +124,14 @@ class MSDeformAttnMergedFunction(Function):
     (both linears of the reference module read the same `query`, ms_deform_attn.py:108-111). The kernels read the two
     column blocks in place and write their gradient in the same layout, so the backward is also one GEMM.
 
-        apply(value, spatial_shapes, level_start_index, reference_points, merged, n_levels, n_points)"""
+        apply(value, spatial_shapes, level_start_index, reference_points, merged, n_levels, n_points)
+
+    `reference_points` as in MSDeformAttnFusedFunction: points or boxes, with a gradient exactly when it requires one."""
 
     @staticmethod
     def forward(ctx, value, value_spatial_shapes, value_level_start_index, reference_points, merged, n_levels, n_points):
         value = _amp_value(value)
-        reference_points = reference_points.float().contiguous()
+        reference_points = _fused_ref(reference_points)
         merged = merged.float().contiguous()
         ctx.lp = (int(n_levels), int(n_points))
         output = _cabi.forward_fused_merged(value, value_spatial_shapes, value_level_start_index, reference_points,
@@ -128,6 +143,7 @@ class MSDeformAttnMergedFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         value, shapes, level_start, ref, merged = ctx.saved_tensors
-        grad_value, grad_merged = _cabi.backward_fused_merged(value, shapes, level_start, ref, merged, *ctx.lp,
-                                                              _grad_output(grad_output, value))
-        return grad_value, None, None, None, grad_merged, None, None
+        want_ref = ctx.needs_input_grad[3]
+        grads = _cabi.backward_fused_merged(value, shapes, level_start, ref, merged, *ctx.lp, _grad_output(grad_output, value),
+                                            ref_grad=want_ref)
+        return grads[0], None, None, grads[2] if want_ref else None, grads[1], None, None

@@ -84,9 +84,10 @@ class MSDeformAttn(nn.Module):
         self.output_proj = nn.Linear(d_value, d_model)
         self._checked_shapes = _cabi.TensorMemo(limit=64)
         self._merged_cache = None   # (key, weight, bias) of _MergedQueryParams
-        # fuse softmax + location arithmetic into the sampling kernel when a fused kernel exists (2-d reference
-        # points, CUDA, fp32/bf16, (L,P) in {(3,4),(1,4)}); results differ from the unfused path only by the
-        # rounding of the softmax normalisation. Set to False to force the reference's op sequence.
+        # fuse softmax + location arithmetic into the sampling kernel when a fused kernel exists (CUDA, fp32 / bf16 /
+        # fp16, D in {32, 64}, (L,P) in {(3,4),(1,4),(4,4)}; 2-d or 4-d reference points, with or without gradient);
+        # results differ from the unfused path only by the rounding of the softmax normalisation and the order of the
+        # reference-point gradient's sum. Set to False to force the reference's op sequence.
         self.fused = True
         self.merge_query_linears = True
         # bias gradients of value_proj / output_proj / the merged query linear through the column-sum kernel
@@ -142,11 +143,10 @@ class MSDeformAttn(nn.Module):
             value = value.masked_fill(input_padding_mask[..., None], float(0))
         value = value.view(N, len_in, M, int(self.ratio * self.d_model) // M)
 
-        # The fused kernels return no gradient for reference_points (a constant grid in the adapter). A caller that learns
-        # its reference points (Deformable-DETR style decoders, ms_deform_attn.py:115-119 differentiates them) takes the
-        # reference's op sequence below, which does.
-        ref_needs_grad = torch.is_grad_enabled() and reference_points.requires_grad
-        if self.fused and not ref_needs_grad and reference_points.dim() == 4 and reference_points.shape[-1] == 2 \
+        # The fused kernels take points [.., 2] and boxes [.., 4] and return a reference-point gradient exactly when
+        # autograd asks for one (Deformable-DETR style decoders learn their reference points, ms_deform_attn.py:115-119);
+        # the adapter's constant grid gets none and launches nothing extra for it.
+        if self.fused and reference_points.dim() == 4 and reference_points.shape[-1] in (2, 4) \
                 and _cabi.fused_supported(value, L, P):
             if self.merge_query_linears:
                 # sampling_offsets and attention_weights read the same query: ONE GEMM over the concatenated weights
