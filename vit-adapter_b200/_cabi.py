@@ -565,6 +565,12 @@ def layernorm_forward(x, weight, bias, eps, out_dtype):
 def layernorm_backward(grad_y, x, weight, stats, grad_residual=None):
     """(grad_x in x.dtype, grad_weight fp32 [C], grad_bias fp32 [C]); grad_residual (x's shape and dtype, contiguous) is
     added into grad_x."""
+    gx, gwb = layernorm_backward_stacked(grad_y, x, weight, stats, grad_residual)
+    return gx, gwb[0], gwb[1]
+
+
+def layernorm_backward_stacked(grad_y, x, weight, stats, grad_residual=None):
+    """layernorm_backward with grad_weight and grad_bias returned as the one fp32 [2, C] buffer the kernel writes."""
     lib = load()
     dev = _check_cuda(grad_y=grad_y, x=x, weight=weight)
     if grad_residual is not None:
@@ -585,7 +591,7 @@ def layernorm_backward(grad_y, x, weight, stats, grad_residual=None):
                                             rows, C, ws.data_ptr(), ws_bytes, _stream())
     if rc != 0:
         _raise(rc, 'adapter_layernorm_backward')
-    return gx, gwb[0], gwb[1]
+    return gx, gwb
 
 
 # --- bias gradient of the adapter's Linears (SURVEY §8(f) N1) ------------------------------------------------------------
@@ -619,10 +625,15 @@ def colsum(x):
 
 
 # --- residual epilogue (SURVEY §8(f) N2) ----------------------------------------------------------------------------------
-def residual_add_supported(res, branch):
+def residual_add_layout_supported(res, branch):
+    """residual_add_supported without its pointer-alignment test (which compiled code defers to run time)."""
     return (res.is_cuda and branch.is_cuda and res.dtype == torch.float32 and branch.dtype in (torch.float32, torch.bfloat16, torch.float16)
             and res.shape == branch.shape and res.is_contiguous() and branch.is_contiguous() and res.numel() > 0
-            and res.numel() % 8 == 0 and res.data_ptr() % 16 == 0 and branch.data_ptr() % 16 == 0)
+            and res.numel() % 8 == 0)
+
+
+def residual_add_supported(res, branch):
+    return residual_add_layout_supported(res, branch) and res.data_ptr() % 16 == 0 and branch.data_ptr() % 16 == 0
 
 
 def residual_add(res, branch):

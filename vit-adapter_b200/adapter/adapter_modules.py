@@ -12,6 +12,10 @@ Differences from the reference, all host-side:
     which costs ~20 tiny kernel launches and makes the tensors' storage change every step (defeating
     MSDeformAttn's cached shape check and CUDA-graph capture).
   * DropPath is implemented here (timm is not a dependency).
+
+Under torch.compile / torch.export the LayerNorm, residual-add and depth-wise conv kernels are reached through the
+msda_b200 custom ops (`_ops.py`). The one compiled-mode difference: the LayerNorm op returns only y, so the pre-norm
+residual uses x itself and its gradient is added by the compiled graph instead of inside the LayerNorm backward kernel.
 """
 from functools import partial
 
@@ -21,6 +25,7 @@ import torch.utils.checkpoint as cp
 
 from .. import _cabi
 from ..functions import linear
+from ..functions.ms_deform_attn_func import _compiled_ops
 from ..modules import MSDeformAttn
 
 
@@ -137,6 +142,8 @@ def apply_norm(norm, x, fused=True):
     tensor directly (torch would write fp32 and cast it again); anything else calls the module as the reference does."""
     out_dtype = _norm_kernel_dtype(norm, x, fused)
     if out_dtype is not None:
+        if torch.compiler.is_compiling():
+            return _compiled_ops().layernorm(x, norm.weight, norm.bias, norm.eps, out_dtype)[0]
         return _LayerNormRows.apply(x, norm.weight, norm.bias, norm.eps, out_dtype, False)
     return norm(x)
 
@@ -144,7 +151,10 @@ def apply_norm(norm, x, fused=True):
 def apply_norm_residual(norm, x, fused=True):
     """(norm(x), x') for the pre-norm residual pattern `x + f(norm(x))` (reference adapter_modules.py:113-116, :145):
     use x' (same values as x) for the residual connection. With the row kernel, the gradient of x' is folded into the
-    LayerNorm backward kernel instead of a separate full-tensor add by autograd."""
+    LayerNorm backward kernel instead of a separate full-tensor add by autograd (not in compiled code: see the module
+    docstring)."""
+    if torch.compiler.is_compiling():
+        return apply_norm(norm, x, fused), x
     out_dtype = _norm_kernel_dtype(norm, x, fused)
     if out_dtype is not None and torch.is_grad_enabled() and x.requires_grad:
         return _LayerNormRows.apply(x, norm.weight, norm.bias, norm.eps, out_dtype, True)
@@ -167,6 +177,11 @@ class _ResidualAdd(torch.autograd.Function):
 
 def residual_add(res, branch, fused=True):
     """`res + branch` (reference adapter_modules.py:113-116); the mixed fp32 + bf16 case goes through the kernel."""
+    if torch.compiler.is_compiling():
+        # the 16-byte alignment of the operands is known only at run time: the op copies a misaligned one
+        if fused and res.dtype != branch.dtype and _cabi.residual_add_layout_supported(res, branch):
+            return _compiled_ops().residual_add(res, branch)
+        return res + branch
     if fused and res.dtype != branch.dtype and _cabi.residual_add_supported(res, branch):
         return _ResidualAdd.apply(res, branch)
     return res + branch
@@ -209,6 +224,8 @@ class DWConv(nn.Module):
         if self.token_kernel and _cabi.dwconv_supported(x, w.to(x.dtype) if w.dtype != x.dtype else w, H, W):
             if w.dtype != x.dtype:  # autocast: activations bf16, parameters fp32
                 w, b = w.to(x.dtype), (b.to(x.dtype) if b is not None else None)
+            if torch.compiler.is_compiling():
+                return _compiled_ops().dwconv(x, w, b, H, W)
             return _DWConvTokens.apply(x, w, b, H, W)
         B, N, C = x.shape
         n = N // 21

@@ -5,11 +5,13 @@ is one cuBLAS GEMM with the bias epilogue, the backward is the same two GEMMs to
 backward differs: grad_bias = column sums of grad_output goes through the two-stage column-sum kernel instead of torch's
 generic reduction (which at [86 016, 768] bf16 runs ~10x off the HBM roofline on B200). State-dict keys, parameter
 dtypes and results (to rounding of the fp32 sum order) are unchanged; anything the kernel does not take calls F.linear.
+Compiled code (torch.compile / torch.export) reaches the same kernel through the `msda_b200::colsum` custom op.
 """
 import torch
 import torch.nn.functional as F
 
 from .. import _cabi
+from .ms_deform_attn_func import _compiled_ops
 
 
 class _LinearColsumBias(torch.autograd.Function):
@@ -39,7 +41,12 @@ class _LinearColsumBias(torch.autograd.Function):
         if ctx.needs_input_grad[1]:
             gw = gy2.t() @ xc.reshape(-1, xc.shape[-1])
         if ctx.needs_input_grad[2]:
-            gb = _cabi.colsum(gy2) if _cabi.colsum_supported(gy2) else gy2.sum(0)
+            if not _cabi.colsum_supported(gy2):
+                gb = gy2.sum(0)
+            elif torch.compiler.is_compiling():
+                gb = _compiled_ops().colsum(gy2)
+            else:
+                gb = _cabi.colsum(gy2)
         return gx, gw, gb
 
 

@@ -9,6 +9,10 @@ AMP: the reference decorates forward with `custom_fwd(cast_inputs=torch.float32)
 autocast everything is up-cast to fp32. That stays the default. `set_amp_value_dtype(torch.bfloat16)`
 opts in to the bf16 I/O kernels under autocast (value / out in bf16, locations and weights fp32,
 fp32 accumulation) — a capability the reference does not have; `torch.float16` does the same for fp16 autocast.
+
+Under torch.compile / torch.export (`torch.compiler.is_compiling()`) the three Functions call the `torch.ops.msda_b200`
+custom ops of `_ops.py` instead of `_cabi`: same kernels, but opaque to the compiler, so `apply` traces without a graph
+break. Eager calls take the `_cabi` path exactly as before.
 """
 import torch
 from torch.autograd import Function
@@ -51,6 +55,12 @@ def _fused_ref(reference_points):
     return ref
 
 
+def _compiled_ops():
+    """torch.ops.msda_b200, registered by importing `_ops` on the first compiled call (eager processes never load it)."""
+    from .. import _ops  # noqa: F401
+    return torch.ops.msda_b200
+
+
 def _coord_dtype(value_dtype):
     return torch.float64 if value_dtype == torch.float64 else torch.float32
 
@@ -66,8 +76,12 @@ class MSDeformAttnFunction(Function):
         sampling_locations = sampling_locations.to(cdt)
         attention_weights = attention_weights.to(cdt)
         ctx.im2col_step = im2col_step
-        output = _cabi.forward(value, value_spatial_shapes, value_level_start_index,
-                               sampling_locations, attention_weights, im2col_step)
+        if torch.compiler.is_compiling():
+            output = _compiled_ops().ms_deform_attn(value, value_spatial_shapes, value_level_start_index,
+                                                    sampling_locations, attention_weights, im2col_step)
+        else:
+            output = _cabi.forward(value, value_spatial_shapes, value_level_start_index,
+                                   sampling_locations, attention_weights, im2col_step)
         ctx.save_for_backward(value, value_spatial_shapes, value_level_start_index,
                               sampling_locations, attention_weights)
         return output
@@ -76,6 +90,10 @@ class MSDeformAttnFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         value, shapes, level_start, loc, attn = ctx.saved_tensors
+        if torch.compiler.is_compiling():
+            grad_value, grad_loc, grad_attn = _compiled_ops().ms_deform_attn_backward(
+                value, shapes, level_start, loc, attn, _grad_output(grad_output, value), ctx.im2col_step)
+            return grad_value, None, None, grad_loc, grad_attn, None
         grad_value, grad_loc, grad_attn = _cabi.backward(
             value, shapes, level_start, loc, attn, _grad_output(grad_output, value), ctx.im2col_step)
         return grad_value, None, None, grad_loc, grad_attn, None
@@ -99,11 +117,17 @@ class MSDeformAttnFusedFunction(Function):
     def forward(ctx, value, value_spatial_shapes, value_level_start_index, reference_points, sampling_offsets,
                 attn_logits):
         value = _amp_value(value)
-        reference_points = _fused_ref(reference_points)
+        compiling = torch.compiler.is_compiling()
+        # (compiled: the op makes its own alignment copy of the reference points, at run time)
+        reference_points = reference_points.float().contiguous() if compiling else _fused_ref(reference_points)
         sampling_offsets = sampling_offsets.float().contiguous()
         attn_logits = attn_logits.float().contiguous()
-        output = _cabi.forward_fused(value, value_spatial_shapes, value_level_start_index, reference_points,
-                                     sampling_offsets, attn_logits)
+        if compiling:
+            output = _compiled_ops().ms_deform_attn_fused(value, value_spatial_shapes, value_level_start_index,
+                                                          reference_points, sampling_offsets, attn_logits)
+        else:
+            output = _cabi.forward_fused(value, value_spatial_shapes, value_level_start_index, reference_points,
+                                         sampling_offsets, attn_logits)
         ctx.save_for_backward(value, value_spatial_shapes, value_level_start_index, reference_points,
                               sampling_offsets, attn_logits)
         return output
@@ -113,8 +137,12 @@ class MSDeformAttnFusedFunction(Function):
     def backward(ctx, grad_output):
         value, shapes, level_start, ref, offsets, logits = ctx.saved_tensors
         want_ref = ctx.needs_input_grad[3]
-        grads = _cabi.backward_fused(value, shapes, level_start, ref, offsets, logits, _grad_output(grad_output, value),
-                                     ref_grad=want_ref)
+        if torch.compiler.is_compiling():
+            grads = _compiled_ops().ms_deform_attn_fused_backward(value, shapes, level_start, ref, offsets, logits,
+                                                                  _grad_output(grad_output, value), want_ref)
+        else:
+            grads = _cabi.backward_fused(value, shapes, level_start, ref, offsets, logits, _grad_output(grad_output, value),
+                                         ref_grad=want_ref)
         grad_value, grad_off, grad_logits = grads[:3]
         return grad_value, None, None, grads[3] if want_ref else None, grad_off, grad_logits
 
@@ -131,11 +159,16 @@ class MSDeformAttnMergedFunction(Function):
     @staticmethod
     def forward(ctx, value, value_spatial_shapes, value_level_start_index, reference_points, merged, n_levels, n_points):
         value = _amp_value(value)
-        reference_points = _fused_ref(reference_points)
+        compiling = torch.compiler.is_compiling()
+        reference_points = reference_points.float().contiguous() if compiling else _fused_ref(reference_points)
         merged = merged.float().contiguous()
         ctx.lp = (int(n_levels), int(n_points))
-        output = _cabi.forward_fused_merged(value, value_spatial_shapes, value_level_start_index, reference_points,
-                                            merged, *ctx.lp)
+        if compiling:
+            output = _compiled_ops().ms_deform_attn_merged(value, value_spatial_shapes, value_level_start_index,
+                                                           reference_points, merged, *ctx.lp)
+        else:
+            output = _cabi.forward_fused_merged(value, value_spatial_shapes, value_level_start_index, reference_points,
+                                                merged, *ctx.lp)
         ctx.save_for_backward(value, value_spatial_shapes, value_level_start_index, reference_points, merged)
         return output
 
@@ -144,6 +177,10 @@ class MSDeformAttnMergedFunction(Function):
     def backward(ctx, grad_output):
         value, shapes, level_start, ref, merged = ctx.saved_tensors
         want_ref = ctx.needs_input_grad[3]
-        grads = _cabi.backward_fused_merged(value, shapes, level_start, ref, merged, *ctx.lp, _grad_output(grad_output, value),
-                                            ref_grad=want_ref)
+        if torch.compiler.is_compiling():
+            grads = _compiled_ops().ms_deform_attn_merged_backward(value, shapes, level_start, ref, merged, *ctx.lp,
+                                                                   _grad_output(grad_output, value), want_ref)
+        else:
+            grads = _cabi.backward_fused_merged(value, shapes, level_start, ref, merged, *ctx.lp,
+                                                _grad_output(grad_output, value), ref_grad=want_ref)
         return grads[0], None, None, grads[2] if want_ref else None, grads[1], None, None
