@@ -128,7 +128,15 @@ __global__ void __launch_bounds__(kLnWarps * 32, 2) adapter_ln_fwd_kernel(const 
     float s = 0.f;
 #pragma unroll
     for (int i = 0; i < VPL; ++i) s += (xv[i][0] + xv[i][1]) + (xv[i][2] + xv[i][3]);
-    const float mean = warp_sum(s) * inv_c;
+    const float m0 = warp_sum(s) * inv_c;
+    // second pass: mean = m0 + mean(x - m0). The row sum's rounding scales with |x|, the correction's with the spread
+    // |x - m0|: a row with a large common offset gets its mean to within the spread's precision, and a constant row gets
+    // exactly its value (so y == beta, as with torch's Welford statistics) instead of an error that 1/sqrt(eps) magnifies
+    float sd = 0.f;
+#pragma unroll
+    for (int i = 0; i < VPL; ++i)
+      if (ok[i]) sd += ((xv[i][0] - m0) + (xv[i][1] - m0)) + ((xv[i][2] - m0) + (xv[i][3] - m0));
+    const float mean = m0 + warp_sum(sd) * inv_c;
     float q = 0.f;
 #pragma unroll
     for (int i = 0; i < VPL; ++i)
