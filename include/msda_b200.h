@@ -10,6 +10,10 @@
  *
  * Conventions
  *   - All tensor pointers are DEVICE pointers to contiguous row-major storage.
+ *   - msda_forward / msda_backward accept any pointer aligned to its element size (else MSDA_E_ALIGN); better
+ *     aligned tensors may take faster kernels, with results within the same rounding bounds. The fused entry points
+ *     need 16-byte aligned value / out / grad_out and 8-byte aligned offsets, but only the element size of a 16-bit
+ *     grad_value.
  *   - The library never allocates or frees tensor memory (the reference allocates with
  *     at::zeros inside C++, ms_deform_attn_cuda.cu:54,121-123). The caller owns every buffer.
  *   - `stream` is a cudaStream_t passed as void*; every call is asynchronous w.r.t. the host,

@@ -14,14 +14,12 @@ u_out is the unit roundoff of the output dtype (2^-8 bf16, 2^-11 f16, 0 when the
 acc bounds the accumulation error (c * u_acc * sum of |terms| for a sum), floor is half the subnormal spacing of the
 output dtype. Each `acc` says where its constant comes from.
 """
-import math
-import re
-
 import pytest
 import torch
 import torch.nn.functional as F
 from torch import nn
 
+from kernel_paths import assert_within, at_offset, kernel, kernels_launched
 from oracle import dwconv_ref, layernorm_ref
 
 pytestmark = pytest.mark.gpu
@@ -34,38 +32,6 @@ SHORT = {torch.float32: 'f32', torch.bfloat16: 'bf16', torch.float16: 'f16', tor
 
 
 # --- helpers -------------------------------------------------------------------------------------------------------------
-def at_offset(t, byte_offset):
-    """A contiguous copy of `t` that starts `byte_offset` bytes into a larger (allocator-aligned) buffer."""
-    es = t.element_size()
-    assert byte_offset % es == 0
-    k = byte_offset // es
-    buf = torch.empty(t.numel() + k + 16, dtype=t.dtype, device=t.device)
-    out = buf[k:k + t.numel()].view(t.shape)
-    out.copy_(t)
-    assert out.is_contiguous() and out.data_ptr() % 16 == byte_offset % 16, (out.data_ptr(), byte_offset)
-    return out
-
-
-def kernels_launched(fn):
-    """(fn's result, names of the CUDA kernels fn launched, in order). Memsets and copies are left out."""
-    from torch.autograd import DeviceType
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-        out = fn()
-        torch.cuda.synchronize()
-    names = [e.name for e in prof.events() if e.device_type == DeviceType.CUDA
-             and not e.name.startswith(('Memset', 'Memcpy', 'memset', 'memcpy'))]
-    return out, names
-
-
-def kernel(name, *args):
-    """Regex for a kernel by template name and arguments, tolerant of the demangler's spacing."""
-    if not args:
-        return re.compile(r'\b%s\s*\(' % name)
-    return re.compile(r'\b%s\s*<\s*%s\s*>' % (name, r'\s*,\s*'.join(re.escape(str(a)) for a in args)))
-
-
 def assert_kernels(names, expected, what):
     """Every expected pattern matched by exactly one launched kernel of this project, and no other such kernel."""
     ours = [n for n in names if 'adapter_' in n]
@@ -73,25 +39,6 @@ def assert_kernels(names, expected, what):
         hits = [n for n in ours if pat.search(n)]
         assert len(hits) == 1, '%s: expected one launch of /%s/, got %s' % (what, pat.pattern, ours)
     assert len(ours) == len(expected), '%s: launched %s, expected %s' % (what, ours, [p.pattern for p in expected])
-
-
-def unit_roundoff(dtype):
-    return {torch.float32: 0.0, torch.float64: 0.0, torch.bfloat16: 2.0 ** -8, torch.float16: 2.0 ** -11}[dtype]
-
-
-def assert_within(out, ref, acc, what):
-    """|out - ref| <= u_out |ref| + (1 + u_out) acc + floor, elementwise, in fp64."""
-    fi = torch.finfo(out.dtype)
-    uo = unit_roundoff(out.dtype)
-    err = (out.double() - ref).abs()
-    bound = uo * ref.abs() + (1.0 + uo) * acc + fi.smallest_normal * fi.eps / 2
-    bad = ~(err <= bound)
-    if bad.any():
-        ratio = torch.where(bound > 0, err / bound, torch.full_like(err, math.inf))
-        i = int(ratio.flatten().argmax())
-        raise AssertionError('%s: %d of %d elements outside the bound; worst at flat index %d: out %r ref %r err %.3e bound %.3e'
-                             % (what, int(bad.sum()), err.numel(), i, float(out.flatten()[i]), float(ref.flatten()[i]),
-                                float(err.flatten()[i]), float(bound.flatten()[i])))
 
 
 def _sms():

@@ -659,8 +659,10 @@ static int backward_fused_body(const char* who, const msda_dims* dims, int dtype
   p.grad_out = grad_out; p.grad_loc = grad_sampling_offsets; p.grad_aw = grad_attn_logits;
   if (int e = fused_ref_params(p, dims, reference_points, ref_batch, ref_levels, ref_dim, offsets_row_stride, logits_row_stride))
     return e;
+  // a 16-bit grad_value needs only its element size: the convert that writes it picks its stores from the alignment
   if (!aligned(value, 16) || !aligned(grad_out, 16) || !aligned(backward_accum(dtype, grad_value, workspace), 16) ||
-      !aligned(sampling_offsets, 8) || !aligned(grad_sampling_offsets, 8) || (ref_grad && !aligned(grad_reference_points, 4)))
+      !aligned(grad_value, elem_size(dtype)) || !aligned(sampling_offsets, 8) || !aligned(grad_sampling_offsets, 8) ||
+      (ref_grad && !aligned(grad_reference_points, 4)))
     return fail(MSDA_E_ALIGN, "%s: misaligned pointer", who);
   if (ref_grad) p.ref_partial = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + ref_partial_offset(dims, dtype));
   const cudaStream_t s = (cudaStream_t)stream;

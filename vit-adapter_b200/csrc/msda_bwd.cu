@@ -507,6 +507,13 @@ __global__ void __launch_bounds__(kThreads) msda_cvt_f32_bf16_kernel(const float
     st_scalar(dst + i, src[i]);
 }
 
+// The same conversion for a grad_value that is not 16-byte aligned: the C ABI only requires the element size.
+template <typename TO>
+__global__ void __launch_bounds__(kThreads) msda_cvt_f32_bf16_scalar_kernel(const float* __restrict__ src, TO* __restrict__ dst, size_t n) {
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+    st_scalar(dst + i, src[i]);
+}
+
 // ---------------------------------------------------------------------------------------------
 // Launchers
 // ---------------------------------------------------------------------------------------------
@@ -604,10 +611,12 @@ static cudaError_t launch_packed_t(const Params& p, int G, bool fused, dim3 grid
 
 template <typename TO>
 static cudaError_t launch_cvt_t(const float* src, void* dst, size_t n, cudaStream_t s) {
-  size_t blocks = (n / 8 + kThreads - 1) / kThreads;
+  const bool vec = reinterpret_cast<uintptr_t>(dst) % 16 == 0;  // 16-byte stores
+  size_t blocks = ((vec ? n / 8 : n) + kThreads - 1) / kThreads;
   if (blocks < 1) blocks = 1;
   if (blocks > 148u * 16u) blocks = 148u * 16u;
-  msda_cvt_f32_bf16_kernel<TO><<<(unsigned)blocks, kThreads, 0, s>>>(src, reinterpret_cast<TO*>(dst), n);
+  if (vec) msda_cvt_f32_bf16_kernel<TO><<<(unsigned)blocks, kThreads, 0, s>>>(src, reinterpret_cast<TO*>(dst), n);
+  else msda_cvt_f32_bf16_scalar_kernel<TO><<<(unsigned)blocks, kThreads, 0, s>>>(src, reinterpret_cast<TO*>(dst), n);
   return cudaGetLastError();
 }
 
